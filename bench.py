@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- control env-steps/s of the batched Go1+PEA step path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--config {2,3,4,5}]     (ours; N>1 under torchrun)
+    python bench.py --gpus N --steps K --warmup W [--config {2,3,4,5}] [--dump-outputs DIR]     (ours; N>1 under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W [--config ...]
 
 One "step" = one control step (action_repeat = 10 physics ticks + task/obs epilogue, finished envs
@@ -41,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree, which may be read-only
 
 CONFIGS = {
     2: dict(name="go1_nosprings_jumping_in_place_pd_4096env", kind="random", envs_per_gpu=4096,
@@ -279,16 +280,17 @@ class Job:
         return None
 
     def step(self, inp):
+        """one bench step; returns what the env hands its caller: (obs, reward, done, infos), views of the env's buffers"""
         env = self.env
         if self.kind == "random":
-            o, r, d, _ = env.step(inp)
-        elif self.kind == "cpg":    # hopf_network.py:241-289, ten 1 ms ticks: qs_cpg_steps
-            self.cpg.drive(env, 10)
-            return
-        else:                       # load_model.py:127-134 with the policy on the device (stochastic, as in PPO rollouts)
-            a = self.policy.predict(self.vn.normalize_obs(self.obs), deterministic=False, generator=self.gen)
-            o, r, d, _ = env.step(a)
-            self.obs = o
+            return env.step(inp)
+        if self.kind == "cpg":      # hopf_network.py:241-289, ten 1 ms ticks: qs_cpg_steps
+            return self.cpg.drive(env, 10)
+        # load_model.py:127-134 with the policy on the device (stochastic, as in PPO rollouts)
+        a = self.policy.predict(self.vn.normalize_obs(self.obs), deterministic=False, generator=self.gen)
+        out = env.step(a)
+        self.obs = out[0]
+        return out
 
     def take_done_count(self):
         """episodes finished since the last call (the env's own rollout statistics, kernel K5)"""
@@ -340,6 +342,32 @@ def preroll(job, L, lib, max_steps, world, dist, dev, min_steps=150):
     return info
 
 
+DUMP_BYTES = 64 * 10**6    # all .npy files of --dump-outputs together
+DUMP_NAMES = {"TimeLimit.truncated": "truncated"}
+
+
+def dump_outputs(out_dir, outputs, seed=0):
+    """Writes what one step returned to its caller (obs, reward, done and the infos tensors) as out_dir/<name>.npy in float32,
+    one row per env.  If all rows exceed DUMP_BYTES, a fixed seeded sample of env rows is written instead, the same rows in
+    every array, and their indices go to env_index.npy (float64)."""
+    import numpy as np
+    import torch
+    o, r, d, infos = outputs
+    arrays = {"obs": o, "reward": r, "done": d, **{DUMP_NAMES.get(k, k): v for k, v in infos.items()}}
+    n = o.shape[0]
+    row_bytes = sum(4 * a[0].numel() for a in arrays.values())
+    budget = DUMP_BYTES - 128 * (len(arrays) + 1)      # .npy headers
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(seed).choice(n, budget // (row_bytes + 8), replace=False))
+        idx = torch.as_tensor(rows, device=o.device)
+        arrays = {k: v.index_select(0, idx) for k, v in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        a = v if isinstance(v, np.ndarray) else v.detach().to(torch.float32).cpu().numpy()
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -387,6 +415,9 @@ def run_ours(args):
     nsteps0 = L.qs_step_count(env._h)
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     urgent = 0
+    # the pre-roll's length follows the computed reset counts: reseeding here keeps the timed steps' random draws the same
+    # for builds whose rounding differs, so that their --dump-outputs can be compared
+    job.gen.manual_seed(4321 + rank)
     barrier()
     t_wall = time.perf_counter()
     host_s = 0.0
@@ -395,7 +426,7 @@ def run_ours(args):
         a = job.next_input()           # inputs resident in HBM before the timed region of the step starts
         ev[i][0].record()
         th = time.perf_counter()
-        job.step(a)
+        last = job.step(a)
         host_s += time.perf_counter() - th
         ev[i][1].record()
     barrier()
@@ -418,6 +449,8 @@ def run_ours(args):
     _lib.check(L.qs_debug_counters(env._h, dbg, None))
     urgent = int(dbg[1])
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:     # before the e2e steps below overwrite the env's buffers
+        dump_outputs(args.dump_outputs, last)
     t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -608,7 +641,12 @@ def main():
     ap.add_argument("--series", action="store_true", help="add the per-step device times to the line")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0's shard) as DIR/<name>.npy, float32, "
+                         f"at most {DUMP_BYTES // 10**6} MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
