@@ -316,6 +316,28 @@ int qs_timing_window(qs_handle h);
  * slice}; synchronises the stream */
 int qs_debug_counters(qs_handle h, int32_t* out4, void* stream);
 
+/* Per-substep trace (what QuadrupedGymEnv.set_sub_step_callback / MonitorState read after every stepSimulation,
+ * quadruped_gym_env.py:152,222-223, utils/monitor_state.py:391-396): every later qs_step, qs_step_host and qs_cpg_steps
+ * writes, for the n_traced envs env_ids_dev[0..n_traced) (device int32, distinct, in [0, N)), the values after each of
+ * its action_repeat physics ticks into trace_dev [action_repeat][QS_TRACE_DIM][n_traced] (device float32, caller-owned;
+ * column j = env env_ids_dev[j]).  Row t of the first index is tick t of the step:
+ *   QS_TR_STATE       37 words in qs_get_state order (pos3 quat4 vlin3 vang3 q12 qd12)
+ *   QS_TR_TAU_MOTOR   12 clipped motor torques applied in that tick (GetMotorTorques)
+ *   QS_TR_TAU_SPRING  12 spring torques applied in that tick
+ *   QS_TR_FOOT_FORCE  4 foot normal forces, 0 for a foot not in contact (GetContactInfo)
+ *   QS_TR_CONTACT     contact word (mask & 15) | invalid << 8 as a float (exact)
+ * With auto_reset, the rows of an env whose episode ends in the step are the ticks of that episode (the NaN / Inf guard
+ * does not clear them).  Resets, settles and qs_debug_ticks write nothing.  The ids are checked on the host (the call
+ * synchronises the device); QS_ERR_ARG when n_traced is not in [1, N] or an id repeats or is out of range.
+ * trace_dev == NULL clears the trace.  Steps without a trace run the same kernels as before the feature existed. */
+#define QS_TRACE_DIM 66
+#define QS_TR_STATE 0
+#define QS_TR_TAU_MOTOR 37
+#define QS_TR_TAU_SPRING 49
+#define QS_TR_FOOT_FORCE 61
+#define QS_TR_CONTACT 65
+int qs_set_substep_trace(qs_handle h, const int32_t* env_ids_dev, int n_traced, float* trace_dev);
+
 /* number of kernels launched by this library since load (bench bookkeeping) */
 int64_t qs_launch_count(void);
 

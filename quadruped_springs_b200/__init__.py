@@ -5,8 +5,9 @@ from .env import (  # noqa: F401
     MotorInterfaceCollection, SensorCollection, TaskCollection,
 )
 from .hopf_network import HopfNetwork  # noqa: F401
-from . import demo, load_model, ops, stats, vec_env  # noqa: F401
+from . import demo, load_model, ops, stats, substep, vec_env  # noqa: F401
+from .substep import SubstepRecorder  # noqa: F401
 from .vec_env import BatchedVecEnv, MlpPolicyTorch, VecNormalizeTorch  # noqa: F401
 
 __all__ = ["BatchedQuadrupedGymEnv", "BatchedQuadruped", "HopfNetwork", "ops", "BatchedVecEnv", "VecNormalizeTorch",
-           "MlpPolicyTorch"]
+           "MlpPolicyTorch", "SubstepRecorder"]

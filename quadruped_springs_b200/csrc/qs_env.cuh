@@ -91,6 +91,45 @@ QS_DEVONLY void load_springs(const DeviceView& D, int env, float* sk, float* sb,
   }
 }
 
+// ---------------------------------------------------------------- per-substep trace (qs_set_substep_trace)
+// buf[t][QS_TRACE_DIM][n_traced]: row t = the values after tick t of the step -- state (store_state's 37 words), the
+// motor and spring torques applied in that tick, foot normal forces (0 off contact), contact word.  A tick handed over
+// to another kernel (TICK_NEEDS_*) is run again by that kernel from the same state, which then owns its row.
+struct SubstepTrace {
+  float* buf;          // nullptr: no trace
+  int32_t* col;        // [N]: the env's column, -1 when it is not traced
+  int n_traced;
+};
+// one env's column of the trace: p = &buf[0][0][col], or nullptr when the env is not traced (or the thread has no env)
+struct TraceColumn {
+  float* p;
+  int w;   // n_traced: distance between two rows
+  QS_DEVONLY float* row(int t, int r) const { return p + (size_t(t) * QS_TRACE_DIM + r) * size_t(w); }
+  QS_DEVONLY void torques(int t, const float* tm, const float* ts) const {
+    if (!p) return;
+#pragma unroll
+    for (int i = 0; i < 12; i++) { *row(t, QS_TR_TAU_MOTOR + i) = tm[i]; *row(t, QS_TR_TAU_SPRING + i) = ts[i]; }
+  }
+  QS_DEVONLY void state(int t, const EnvState<float>& st, const ContactState<float>& cs, float dt) const {
+    if (!p) return;
+#pragma unroll
+    for (int i = 0; i < 3; i++) *row(t, QS_TR_STATE + i) = st.pos[i];
+#pragma unroll
+    for (int i = 0; i < 4; i++) *row(t, QS_TR_STATE + 3 + i) = st.quat[i];
+#pragma unroll
+    for (int i = 0; i < 3; i++) { *row(t, QS_TR_STATE + 7 + i) = st.vlin[i]; *row(t, QS_TR_STATE + 10 + i) = st.vang[i]; }
+#pragma unroll
+    for (int i = 0; i < 12; i++) { *row(t, QS_TR_STATE + 13 + i) = st.q[i]; *row(t, QS_TR_STATE + 25 + i) = st.qd[i]; }
+#pragma unroll
+    for (int k = 0; k < 4; k++) *row(t, QS_TR_FOOT_FORCE + k) = (cs.mask >> k) & 1 ? cs.lam_n[k] / dt : 0.f;
+    *row(t, QS_TR_CONTACT) = float((cs.mask & 15) | (cs.invalid << 8));
+  }
+};
+QS_DEVONLY TraceColumn trace_column(const SubstepTrace& tr, int env, bool live) {
+  const int c = live ? tr.col[env] : -1;
+  return TraceColumn{c >= 0 ? tr.buf + c : nullptr, tr.n_traced};
+}
+
 // ApplyAction + stepSimulation for ticks [t0, n_ticks) (quadruped_gym_env.py:207-219).
 // cmd = desired joint angles (PD) or torques (TORQUE).  Returns n_ticks when all ticks ran,
 // or the index of the tick that needs another solver (state untouched by that tick; *why =
@@ -101,13 +140,14 @@ QS_DEVONLY void load_springs(const DeviceView& D, int env, float* sk, float* sb,
 constexpr int QS_BLOCK = 128;
 using StepScratch = Scratch<float, QS_BLOCK>;
 
-template <bool kContacts, bool kEM>
+// kTrace: each tick this thread completes goes to its trace column `tc`.
+template <bool kContacts, bool kEM, bool kTrace = false>
 __device__ __forceinline__ int run_ticks(EnvState<float>& st, ContactState<float>& cs, const float* cmd,
                                          bool torque_mode, int t0, int n_ticks, int env, const DeviceView& D,
                                          const EnvCfg& C, const RobotConst& RC, const ModelConstT<float>& M,
                                          const ModelLegPairsT<float>& M2, const SolverConst& SC, float* tau_m /*12 out*/,
                                          float* tau_s /*12 out*/, bool detect_invalid_last, const StepScratch& scr, int* why,
-                                         bool skip = false) {
+                                         TraceColumn tc = TraceColumn{nullptr, 0}, bool skip = false) {
   const float mu = D.mu[env];
   const bool custom = D.custom_gains[env] != 0;
   {  // the motor command and the springs are the same for every tick: parked in the scratch, read back by each tick
@@ -141,6 +181,7 @@ __device__ __forceinline__ int run_ticks(EnvState<float>& st, ContactState<float
         sr[j] = *static_cast<const volatile float*>(&scr.park(18 + j));
       }
       tick_torques(st, c12, torque_mode, env, D, C, RC, sk, sb, sr, tau, tm, ts, custom);
+      if constexpr (kTrace) tc.torques(t, tm, ts);   // (rewritten by the next kernel if this tick is handed over)
       if (t == n_ticks - 1) {
         kept = true;
 #pragma unroll
@@ -149,6 +190,7 @@ __device__ __forceinline__ int run_ticks(EnvState<float>& st, ContactState<float
       const int r = physics_tick<float, kContacts, QS_BLOCK, kEM>(st, tau, mu, cs, M, SC, detect_invalid_last && (t == n_ticks - 1), scr,
                                                              EnvModelRef{D.model, D.n, env}, &M2);
       if (r != TICK_DONE) { bail = t; *why = r; }
+      else if constexpr (kTrace) tc.state(t, st, cs, SC.dt);
     }
   }
   if (kept) {
@@ -158,12 +200,15 @@ __device__ __forceinline__ int run_ticks(EnvState<float>& st, ContactState<float
   return bail;
 }
 
-// same loop on the general solver (joint limits, every collision shape); rare path
-template <bool kEM>
+// same loop on the general solver (joint limits, every collision shape); rare path.  The traced variant takes the env's
+// trace column as one more argument (`tc`, a pack so that the default variant keeps its calling sequence).
+template <bool kEM, bool kTrace = false, typename... Col>
 __device__ __noinline__ void run_ticks_general(EnvState<float>& st, ContactState<float>& cs, const float* cmd,
                                                bool torque_mode, int t0, int n_ticks, int env, const DeviceView& D,
                                                const EnvCfg& C, const RobotConst& RC, const ModelConstT<float>& M,
-                                               const SolverConst& SC, float* tau_m, float* tau_s, float* dl, int dl_stride) {
+                                               const SolverConst& SC, float* tau_m, float* tau_s, float* dl, int dl_stride,
+                                               Col... tc) {
+  static_assert(sizeof...(Col) == (kTrace ? 1 : 0), "the traced variant takes one TraceColumn");
   const float mu = D.mu[env];
   const bool custom = D.custom_gains[env] != 0;
   float sk[3], sb[3], sr[3];
@@ -172,6 +217,11 @@ __device__ __noinline__ void run_ticks_general(EnvState<float>& st, ContactState
     float tau[12];
     tick_torques(st, cmd, torque_mode, env, D, C, RC, sk, sb, sr, tau, tau_m, tau_s, custom);
     physics_tick_general<float, kEM>(st, tau, mu, cs, M, SC, EnvModelRef{D.model, D.n, env}, dl, dl_stride);
+    if constexpr (kTrace) {
+      const TraceColumn c[] = {tc...};
+      c[0].torques(t, tau_m, tau_s);
+      c[0].state(t, st, cs, SC.dt);
+    }
   }
 }
 

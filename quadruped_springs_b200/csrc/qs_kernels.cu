@@ -13,6 +13,8 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <type_traits>
+#include <vector>
 
 #include "qs_env.cuh"
 #include "qs_model_host.h"
@@ -353,6 +355,7 @@ struct qs_env {
   cudaEvent_t ev_late;
   float* term_obs;     // caller-owned, optional (qs_set_terminal_obs)
   float* dev_demo;     // demonstration actions of the *_DEMO tasks (qs_set_demo)
+  SubstepTrace trace;  // qs_set_substep_trace: caller-owned rows, column map in the pool (trace.buf == nullptr: off)
   bool was_reset;
   // CUDA-event ring around k_step launches (roofline timing of the dominant kernel)
   static constexpr int kRing = 512;
@@ -534,7 +537,7 @@ int qs_create(const qs_config* cfg, int n_envs, int device, qs_handle* out) {
 
   // one pool for all SoA arrays (4-byte elements), 256 B aligned segments
   const size_t n = size_t(n_envs);
-  const size_t rows = 37 + 12 + 12 + 12 + 12 + 9 + 1 + 4 + 1 + QS_TASK_DIM + 12 + 48 + 1 + 1 + 1 + QS_STATS_DIM + 1 + 3 + 12 + 1 + 1 + 1 + 2 + 1 + 14 + EM_ROWS + 8 + QS_SLOTS * (SLOT_ROWS + 1 + 1);
+  const size_t rows = 37 + 12 + 12 + 12 + 12 + 9 + 1 + 4 + 1 + QS_TASK_DIM + 12 + 48 + 1 + 1 + 1 + QS_STATS_DIM + 1 + 3 + 12 + 1 + 1 + 1 + 2 + 1 + 14 + EM_ROWS + 8 + QS_SLOTS * (SLOT_ROWS + 1 + 1) + 1;
   // rows of one array are contiguous with stride n floats; each array starts 256 B aligned
   h->pool_bytes = rows * n * 4 + 64 * 256;
   cudaError_t e = cudaMalloc(&h->pool, h->pool_bytes);
@@ -563,6 +566,7 @@ int qs_create(const qs_config* cfg, int n_envs, int device, qs_handle* out) {
   D.rest_active = (int32_t*)carve(1); D.rest = (float*)carve(14);
   D.model = (float*)carve(EM_ROWS); D.mass_draw = (float*)carve(8);
   D.slot = (float*)carve(QS_SLOTS * SLOT_ROWS); D.slot_contact = (int32_t*)carve(QS_SLOTS); D.slot_epoch = (uint32_t*)carve(QS_SLOTS);
+  h->trace.col = (int32_t*)carve(1);
   if (size_t(p - static_cast<char*>(h->pool)) > h->pool_bytes) { cudaFree(h->pool); delete h; return fail(QS_ERR_STATE, "pool overflow"); }
   {
     // settle conveyor: window = one wave of settle blocks (2 per SM); the queue holds every ring entry
@@ -637,12 +641,16 @@ int qs_create(const qs_config* cfg, int n_envs, int device, qs_handle* out) {
   }
   {
     const int max_smem = int(smem_of(256));
-    e = cudaFuncSetAttribute(k_step<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    e = cudaFuncSetAttribute(k_step<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_reset<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_reset<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_settle_urgent<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_settle_urgent<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_settle_slice<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
@@ -962,15 +970,27 @@ static int step_impl(qs_handle h, const float* actions, float* obs, float* rewar
   io.stamps = h->stamps + 4 * slot;
   io.flight_cap = h->flight_cap;
   CUDA_TRY(rec_timing(h->ev0[slot], s, capturing));
+  // the tick kernels' instantiation: <mass randomizer, substep trace>
+  const SubstepTrace tr = h->trace;
+  auto tick_kernels = [&](auto launch) {
+    using T = std::true_type;
+    using F = std::false_type;
+    if (h->args.C.mass_randomizer) { if (tr.buf) launch(T{}, T{}); else launch(T{}, F{}); }
+    else { if (tr.buf) launch(F{}, T{}); else launch(F{}, F{}); }
+  };
   k_pre<<<grid_for(h->n, 256), 256, 0, s>>>(h->args, io);
   g_launches += 1;
-  if (h->args.C.mass_randomizer) k_step<true><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io); else k_step<false><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io);
+  tick_kernels([&](auto em, auto trace) {
+    k_step<decltype(em)::value, decltype(trace)::value><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io, tr);
+  });
   if (h->cfg.auto_reset) {
     // conveyor, early slice: on the second stream, next to k_step_contact (about half a wave of blocks)
     if (int e = launch_conveyor(h, s, 0, 0)) return e;
     CUDA_TRY(cudaEventRecord(h->ev_fork0, s));
   }
-  if (h->args.C.mass_randomizer) k_step_contact<true><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io); else k_step_contact<false><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io);
+  tick_kernels([&](auto em, auto trace) {
+    k_step_contact<decltype(em)::value, decltype(trace)::value><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io, tr);
+  });
   g_launches += 1;
   // The epilogue of every env whose ticks are done (all but the general solver's).  With host buffers it runs here, so
   // that the bulk of the results can leave for the host while k_step_slow and the late slice run.  With device buffers
@@ -1009,7 +1029,9 @@ static int step_impl(qs_handle h, const float* actions, float* obs, float* rewar
   // settle slice, which starts once every block of k_step_slow has been placed and runs next to it.  (Round 1 launched
   // the slice on a second stream: when the hardware placed it first, which it did on the three steps that follow a host
   // synchronisation, the general-solver blocks waited for the whole slice, +1 ms; a high-priority stream made it worse.)
-  if (h->args.C.mass_randomizer) k_step_slow<true><<<grid_for(h->n, 64), 64, 0, s>>>(h->args, io, h->slow_spread); else k_step_slow<false><<<grid_for(h->n, 64), 64, 0, s>>>(h->args, io, h->slow_spread);
+  tick_kernels([&](auto em, auto trace) {
+    k_step_slow<decltype(em)::value, decltype(trace)::value><<<grid_for(h->n, 64), 64, 0, s>>>(h->args, io, h->slow_spread, tr);
+  });
   g_launches += 1;
   if (finish_late) {
     cudaLaunchConfig_t cfg = {};
@@ -1149,6 +1171,31 @@ int qs_set_demo(qs_handle h, const float* actions, int length) {
   h->args.C.demo = h->dev_demo;
   h->args.C.demo_len = length;
   drop_graphs(h);   // the kernel arguments are baked into the captured nodes
+  return QS_OK;
+}
+
+int qs_set_substep_trace(qs_handle h, const int32_t* env_ids, int n_traced, float* trace) {
+  if (!h) return fail(QS_ERR_ARG, "handle is NULL");
+  CUDA_TRY(cudaSetDevice(h->device));
+  CUDA_TRY(cudaDeviceSynchronize());  // no step may still be reading the old map or writing the old rows
+  std::vector<int32_t> col;
+  if (trace) {
+    if (n_traced < 1 || n_traced > h->n) return fail(QS_ERR_ARG, "n_traced must be in [1, N]");
+    if (!env_ids) return fail(QS_ERR_ARG, "env_ids is NULL");
+    std::vector<int32_t> ids(size_t(n_traced), 0);
+    CUDA_TRY(cudaMemcpy(ids.data(), env_ids, ids.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    col.assign(size_t(h->n), -1);
+    for (int j = 0; j < n_traced; j++) {
+      const int32_t e = ids[size_t(j)];
+      if (e < 0 || e >= h->n) return fail(QS_ERR_ARG, "env id " + std::to_string(e) + " out of range");
+      if (col[size_t(e)] >= 0) return fail(QS_ERR_ARG, "env id " + std::to_string(e) + " given twice");
+      col[size_t(e)] = j;
+    }
+  }
+  if (trace) CUDA_TRY(cudaMemcpy(h->trace.col, col.data(), col.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  h->trace.buf = trace;
+  h->trace.n_traced = trace ? n_traced : 0;
+  drop_graphs(h);   // the trace is a kernel argument of the captured nodes
   return QS_OK;
 }
 

@@ -915,9 +915,11 @@ k_pre(const __grid_constant__ KernelArgs A, const StepIO io) {
 // -------------------------------------------------------------------- K1: step, flight part
 // The envs with no foot on the ground (dense warps: thread i takes flight_list[i]): flight variant of the tick, no
 // foot-contact code.  An env that reaches the ground goes on to k_step_contact as of the start of that tick.
-template <bool kEM>
+// kTrace (all three tick kernels): the variant launched while a substep trace is set (qs_set_substep_trace); `tr` is
+// read by that variant only
+template <bool kEM, bool kTrace>
 __global__ void __launch_bounds__(256, 1)
-k_step(const __grid_constant__ KernelArgs A, const StepIO io) {
+k_step(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace tr) {
   const int tid = blockIdx.x * blockDim.x + threadIdx.x;
   const DeviceView& D = A.D;
   const EnvCfg& C = A.C;
@@ -941,8 +943,8 @@ k_step(const __grid_constant__ KernelArgs A, const StepIO io) {
   extern __shared__ __align__(16) float qs_smem[];
   const StepScratch scr{qs_smem, QS_BLOCK, int(threadIdx.x)};
   int why;
-  const int t_done = run_ticks<false, kEM>(st, cs, cmd, torque_mode, 0, C.action_repeat, env, D, C, A.RC, A.M, A.M2, A.SC, tau_m, tau_s,
-                                      true, scr, &why);
+  const int t_done = run_ticks<false, kEM, kTrace>(st, cs, cmd, torque_mode, 0, C.action_repeat, env, D, C, A.RC, A.M, A.M2, A.SC, tau_m,
+                                              tau_s, true, scr, &why, kTrace ? trace_column(tr, env, live) : TraceColumn{nullptr, 0});
   if (!live) return;
   if (t_done < C.action_repeat) {
     park_env(A, io, env, st, cs, cmd, t_done, why == TICK_NEEDS_GENERAL ? io.slow_list : io.contact_list);
@@ -954,9 +956,9 @@ k_step(const __grid_constant__ KernelArgs A, const StepIO io) {
 // -------------------------------------------------------------------- K1a: envs with foot contacts
 // Resumes the envs the flight kernel handed over (dense warps: thread i takes contact_list[i]) with
 // the full fast tick; joint limits / body contacts still go on to k_step_slow.
-template <bool kEM>
+template <bool kEM, bool kTrace>
 __global__ void __launch_bounds__(256, 1)
-k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io) {
+k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace tr) {
   const int tid = blockIdx.x * blockDim.x + threadIdx.x;
   const DeviceView& D = A.D;
   const EnvCfg& C = A.C;
@@ -975,8 +977,9 @@ k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io) {
   extern __shared__ __align__(16) float qs_smem[];
   const StepScratch scr{qs_smem, QS_BLOCK, int(threadIdx.x)};
   int why;
-  const int t_done = run_ticks<true, kEM>(st, cs, cmd, torque_mode, D.resume_tick[env], C.action_repeat, env, D, C, A.RC, A.M, A.M2,
-                                     A.SC, tau_m, tau_s, true, scr, &why);
+  const int t_done = run_ticks<true, kEM, kTrace>(st, cs, cmd, torque_mode, D.resume_tick[env], C.action_repeat, env, D, C, A.RC, A.M,
+                                             A.M2, A.SC, tau_m, tau_s, true, scr, &why,
+                                             kTrace ? trace_column(tr, env, live) : TraceColumn{nullptr, 0});
   if (!live) return;
   if (t_done < C.action_repeat) {
     park_env(A, io, env, st, cs, cmd, t_done, io.slow_list);
@@ -986,9 +989,9 @@ k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io) {
 }
 
 // -------------------------------------------------------------------- K1b: general-solver continuation
-template <bool kEM>
+template <bool kEM, bool kTrace>
 __global__ void __launch_bounds__(64)
-k_step_slow(const __grid_constant__ KernelArgs A, const StepIO io, int spread) {
+k_step_slow(const __grid_constant__ KernelArgs A, const StepIO io, int spread, const SubstepTrace tr) {
   // Programmatic dependent launch: the late settle slice follows in the same stream and may start as soon as every block
   // of this grid has been placed (has got here or exited), not when the grid is complete.  That ordering is the point: the
   // slice fills every SM, and when the hardware happened to place it first (two streams racing), the few latency-bound
@@ -1018,8 +1021,12 @@ k_step_slow(const __grid_constant__ KernelArgs A, const StepIO io, int spread) {
   for (int i = 0; i < 12; i++) cmd[i] = D.cmd[i * n + env];
   const bool torque_mode = !A.C.is_rl && A.C.control_mode == QS_CTRL_TORQUE;
   __shared__ float dl_sm[12 * 64];   // the solver's per-leg vector delta (qs_physics.cuh GenRow), one column per thread
-  run_ticks_general<kEM>(st, cs, cmd, torque_mode, D.resume_tick[env], A.C.action_repeat, env, D, A.C, A.RC, A.M, A.SC,
-                    tau_m, tau_s, dl_sm + threadIdx.x, 64);
+  if constexpr (kTrace)
+    run_ticks_general<kEM, true>(st, cs, cmd, torque_mode, D.resume_tick[env], A.C.action_repeat, env, D, A.C, A.RC, A.M, A.SC,
+                                 tau_m, tau_s, dl_sm + threadIdx.x, 64, trace_column(tr, env, true));
+  else
+    run_ticks_general<kEM>(st, cs, cmd, torque_mode, D.resume_tick[env], A.C.action_repeat, env, D, A.C, A.RC, A.M, A.SC,
+                      tau_m, tau_s, dl_sm + threadIdx.x, 64);
   // The epilogue of these envs runs here (not in k_finish): this kernel ends well before the late settle slice it runs
   // next to, while a kernel launched after it would have to wait for that slice.
   D.work[1 * n + env] += uint32_t(cs.work_contacts);

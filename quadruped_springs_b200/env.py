@@ -560,6 +560,7 @@ class BatchedQuadrupedGymEnv:
         self._trunc = torch.zeros(n, dtype=torch.uint8, device=dev)
         self._last_host_obs = None      # where the latest observation lives when it came through the host path
         self.sub_step_callback = None
+        self._trace = self._trace_ids = None
         self.robot_desired_state = None
         if self.verbose > 0:
             self.print_info()
@@ -755,7 +756,35 @@ class BatchedQuadrupedGymEnv:
 
     def set_sub_step_callback(self, callback):
         raise NotImplementedError("per-substep Python callbacks cannot run inside the fused step kernel "
-                                  "(SURVEY.md section 5); read the state tensors between steps instead")
+                                  "(SURVEY.md section 5); set_substep_trace records every substep instead")
+
+    def set_substep_trace(self, env_ids):
+        """Per-substep trace of the envs `env_ids` (qs_set_substep_trace): what a sub_step_callback reading the Quadruped
+        accessors after every stepSimulation would see (quadruped_gym_env.py:222-223).  Returns the float32 tensor
+        [action_repeat, 66, len(env_ids)] that every later step() rewrites: row t = the values after tick t of that step,
+        column j = env env_ids[j]; rows 0-36 state (get_state order), 37-48 motor torque, 49-60 spring torque, 61-64 foot
+        normal force (0 off contact), 65 contact word (mask | invalid << 8, exact as a float).  Under auto_reset, the
+        rows of an env whose episode ended in the step are the ticks of that episode.  None clears the trace; the last
+        buffer is then left as it is.  See substep.SubstepRecorder for a recording over many steps."""
+        if env_ids is None:
+            _lib.check(self._L.qs_set_substep_trace(self._h, None, 0, None))
+            self._trace = self._trace_ids = None
+            return None
+        ids = torch.as_tensor(env_ids)
+        if ids.dtype not in (torch.int32, torch.int64) or ids.dim() != 1:
+            raise ValueError(f"env_ids must be a 1-D integer sequence, got {ids.dtype} of shape {tuple(ids.shape)}")
+        host = ids.cpu()
+        if host.numel() == 0:
+            raise ValueError("env_ids is empty (set_substep_trace(None) clears the trace)")
+        if int(host.min()) < 0 or int(host.max()) >= self.num_envs:
+            raise ValueError(f"env_ids must lie in [0, {self.num_envs})")
+        if host.unique().numel() != host.numel():
+            raise ValueError("env_ids must be distinct")
+        ids = ids.to(device=self.device, dtype=torch.int32).contiguous()
+        buf = torch.full((self._action_repeat, _lib.QS_TRACE_DIM, ids.numel()), float("nan"), device=self.device)
+        _lib.check(self._L.qs_set_substep_trace(self._h, _p(ids), ids.numel(), _p(buf)))
+        self._trace, self._trace_ids = buf, ids      # the library writes into them: keep them alive
+        return buf
 
     def rollout_stats(self):
         """per-shard statistics vector (kernel K5); see stats.gather_rollout_stats"""
