@@ -338,6 +338,25 @@ int qs_debug_counters(qs_handle h, int32_t* out4, void* stream);
 #define QS_TR_CONTACT 65
 int qs_set_substep_trace(qs_handle h, const int32_t* env_ids_dev, int n_traced, float* trace_dev);
 
+/* Quadruped.apply_external_force (quadruped.py:338-343) for the batch: a push on the base, applied inside the step
+ * kernels tick by tick.  wrench_dev [QS_EXT_DIM][N] and ticks_dev [N] are caller-owned device buffers, component-major
+ * like the qs_state_ptrs arrays.  Env i's push is the force F = wrench rows 0-2 (world frame, N) at the point p = rows
+ * 3-5 (base frame, from the base position GetBasePosition, m): in each tick it acts on, it is Bullet's
+ * applyExternalForce(robot, -1, F, pos + R p, WORLD_FRAME) made before that stepSimulation, the moment recomputed from
+ * that tick's orientation.  ticks_dev[i] = n is the number of physics ticks the push still lasts:
+ *   qs_step / qs_step_host / qs_cpg_steps  tick t (0-based) of the step's R = action_repeat ticks is pushed iff t < n
+ *                                          at the start of the step; after the step n -= min(n, R), and with auto_reset
+ *                                          n = 0 for an env whose episode ended in the step (NaN / Inf guard included)
+ *   qs_reset / qs_reset_host / qs_reset_to_state  n = 0 for the reset envs
+ *   qs_debug_ticks                         the same rule over its n_ticks
+ *   settles (the conveyor's included)      never pushed, consume nothing
+ * The library decrements and clears ticks_dev; between steps the caller may write new values into both buffers without
+ * another call.  An env with n = 0 runs exactly the arithmetic of an unpushed step.  Both NULL detaches the buffers (the
+ * steps run the same kernels as before the feature existed); QS_ERR_ARG when exactly one is NULL.  Attaching or
+ * detaching synchronises the device and drops the captured step graphs. */
+#define QS_EXT_DIM 6   /* rows: force xyz (world, N), point xyz (base frame, from the base position, m) */
+int qs_set_external_force(qs_handle h, float* wrench_dev /*[QS_EXT_DIM][N]*/, int32_t* ticks_dev /*[N]*/);
+
 /* number of kernels launched by this library since load (bench bookkeeping) */
 int64_t qs_launch_count(void);
 

@@ -23,6 +23,7 @@ QS_TASK_DIM = 48
 QS_STATS_DIM = 16
 QS_STATE_DIM = 37
 QS_TRACE_DIM = 66   # row of the per-substep trace (qs_set_substep_trace)
+QS_EXT_DIM = 6      # rows of the push wrench (qs_set_external_force): force xyz (world, N), point xyz (base frame, m)
 
 
 class QsConfig(C.Structure):
@@ -114,6 +115,7 @@ EXPORTS = {
     "qs_apply_masses": (C.c_int, [C.c_void_p, C.c_void_p]),
     "qs_set_demo": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "qs_set_substep_trace": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "qs_set_external_force": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "qs_reset_to_state": (C.c_int, [C.c_void_p] * 5),
     "qs_reset_host": (C.c_int, [C.c_void_p] * 4),
     "qs_set_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -130,6 +130,35 @@ QS_DEVONLY TraceColumn trace_column(const SubstepTrace& tr, int env, bool live) 
   return TraceColumn{c >= 0 ? tr.buf + c : nullptr, tr.n_traced};
 }
 
+// ---------------------------------------------------------------- external push on the base (qs_set_external_force)
+// Caller-owned: wrench[QS_EXT_DIM][N] (force xyz, world frame, N; point xyz, base frame from the base position, m) and
+// ticks[N], the ticks the push still lasts.  Every kernel that runs ticks of a step reads the count as of the start of
+// the step (k_ext_countdown consumes it once the step is over), so a tick handed over to another kernel is pushed once.
+struct ExtForce {
+  const float* wrench;   // nullptr: no push buffer
+  int32_t* ticks;
+};
+// one env's push for the ticks of this step: tick t is pushed iff t < n
+struct ExtPush {
+  ExtWrench<float> w;
+  int n;
+  QS_DEVONLY const ExtWrench<float>* at(int t) const { return t < n ? &w : nullptr; }
+};
+QS_DEVONLY ExtPush ext_push(const ExtForce& ef, int env, int n_envs) {
+  ExtPush e;
+  e.n = ef.ticks[env];
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    e.w.f[i] = e.n > 0 ? ef.wrench[size_t(i) * n_envs + env] : 0.f;
+    e.w.p[i] = e.n > 0 ? ef.wrench[size_t(3 + i) * n_envs + env] : 0.f;
+  }
+  return e;
+}
+// (the variadic tail of run_ticks_general: the trace column first, the push last)
+template <typename A, typename... R> QS_DEVONLY A first_of(A a, R...) { return a; }
+template <typename A> QS_DEVONLY A last_of(A a) { return a; }
+template <typename A, typename B, typename... R> QS_DEVONLY auto last_of(A, B b, R... r) { return last_of(b, r...); }
+
 // ApplyAction + stepSimulation for ticks [t0, n_ticks) (quadruped_gym_env.py:207-219).
 // cmd = desired joint angles (PD) or torques (TORQUE).  Returns n_ticks when all ticks ran,
 // or the index of the tick that needs another solver (state untouched by that tick; *why =
@@ -140,14 +169,15 @@ QS_DEVONLY TraceColumn trace_column(const SubstepTrace& tr, int env, bool live) 
 constexpr int QS_BLOCK = 128;
 using StepScratch = Scratch<float, QS_BLOCK>;
 
-// kTrace: each tick this thread completes goes to its trace column `tc`.
-template <bool kContacts, bool kEM, bool kTrace = false>
+// kTrace: each tick this thread completes goes to its trace column `tc`.  kExt: `push` acts on the ticks it covers.
+template <bool kContacts, bool kEM, bool kTrace = false, bool kExt = false>
 __device__ __forceinline__ int run_ticks(EnvState<float>& st, ContactState<float>& cs, const float* cmd,
                                          bool torque_mode, int t0, int n_ticks, int env, const DeviceView& D,
                                          const EnvCfg& C, const RobotConst& RC, const ModelConstT<float>& M,
                                          const ModelLegPairsT<float>& M2, const SolverConst& SC, float* tau_m /*12 out*/,
                                          float* tau_s /*12 out*/, bool detect_invalid_last, const StepScratch& scr, int* why,
-                                         TraceColumn tc = TraceColumn{nullptr, 0}, bool skip = false) {
+                                         TraceColumn tc = TraceColumn{nullptr, 0}, bool skip = false,
+                                         const ExtPush& push = ExtPush{}) {
   const float mu = D.mu[env];
   const bool custom = D.custom_gains[env] != 0;
   {  // the motor command and the springs are the same for every tick: parked in the scratch, read back by each tick
@@ -187,8 +217,9 @@ __device__ __forceinline__ int run_ticks(EnvState<float>& st, ContactState<float
 #pragma unroll
         for (int i = 0; i < 12; i++) { keep[i] = tm[i]; keep[12 + i] = ts[i]; }
       }
-      const int r = physics_tick<float, kContacts, QS_BLOCK, kEM>(st, tau, mu, cs, M, SC, detect_invalid_last && (t == n_ticks - 1), scr,
-                                                             EnvModelRef{D.model, D.n, env}, &M2);
+      const int r = physics_tick<float, kContacts, QS_BLOCK, kEM, kExt>(st, tau, mu, cs, M, SC, detect_invalid_last && (t == n_ticks - 1),
+                                                                   scr, EnvModelRef{D.model, D.n, env}, &M2,
+                                                                   kExt ? push.at(t) : nullptr);
       if (r != TICK_DONE) { bail = t; *why = r; }
       else if constexpr (kTrace) tc.state(t, st, cs, SC.dt);
     }
@@ -201,14 +232,15 @@ __device__ __forceinline__ int run_ticks(EnvState<float>& st, ContactState<float
 }
 
 // same loop on the general solver (joint limits, every collision shape); rare path.  The traced variant takes the env's
-// trace column as one more argument (`tc`, a pack so that the default variant keeps its calling sequence).
-template <bool kEM, bool kTrace = false, typename... Col>
+// trace column as one more argument, the pushed variant the env's ExtPush after it (`x`, a pack so that the default
+// variant keeps its calling sequence).
+template <bool kEM, bool kTrace = false, bool kExt = false, typename... Extra>
 __device__ __noinline__ void run_ticks_general(EnvState<float>& st, ContactState<float>& cs, const float* cmd,
                                                bool torque_mode, int t0, int n_ticks, int env, const DeviceView& D,
                                                const EnvCfg& C, const RobotConst& RC, const ModelConstT<float>& M,
                                                const SolverConst& SC, float* tau_m, float* tau_s, float* dl, int dl_stride,
-                                               Col... tc) {
-  static_assert(sizeof...(Col) == (kTrace ? 1 : 0), "the traced variant takes one TraceColumn");
+                                               Extra... x) {
+  static_assert(sizeof...(Extra) == int(kTrace) + int(kExt), "one TraceColumn when traced, then one ExtPush when pushed");
   const float mu = D.mu[env];
   const bool custom = D.custom_gains[env] != 0;
   float sk[3], sb[3], sr[3];
@@ -216,11 +248,15 @@ __device__ __noinline__ void run_ticks_general(EnvState<float>& st, ContactState
   for (int t = t0; t < n_ticks; t++) {
     float tau[12];
     tick_torques(st, cmd, torque_mode, env, D, C, RC, sk, sb, sr, tau, tau_m, tau_s, custom);
-    physics_tick_general<float, kEM>(st, tau, mu, cs, M, SC, EnvModelRef{D.model, D.n, env}, dl, dl_stride);
+    if constexpr (kExt)
+      physics_tick_general<float, kEM, true>(st, tau, mu, cs, M, SC, EnvModelRef{D.model, D.n, env}, dl, dl_stride,
+                                             last_of(x...).at(t));
+    else
+      physics_tick_general<float, kEM>(st, tau, mu, cs, M, SC, EnvModelRef{D.model, D.n, env}, dl, dl_stride);
     if constexpr (kTrace) {
-      const TraceColumn c[] = {tc...};
-      c[0].torques(t, tau_m, tau_s);
-      c[0].state(t, st, cs, SC.dt);
+      const TraceColumn c0 = first_of(x...);
+      c0.torques(t, tau_m, tau_s);
+      c0.state(t, st, cs, SC.dt);
     }
   }
 }

@@ -104,6 +104,7 @@ template <typename T> struct DebugArgs {
   ModelLegPairsT<T> M2;
   SolverConst SC;
   int mass_randomizer;
+  ExtForce ext;   // the attached push buffer (ext.ticks == nullptr: none); counted down by n_ticks like a step
 };
 template <typename T>
 __global__ void __launch_bounds__(64)
@@ -129,11 +130,17 @@ k_debug_ticks(const __grid_constant__ DebugArgs<T> A, const float* __restrict__ 
   const T mu = T(D.mu[env]);
   extern __shared__ __align__(16) unsigned char qs_smem_raw[];
   const Scratch<T> scr{reinterpret_cast<T*>(qs_smem_raw), int(blockDim.x), int(threadIdx.x)};
+  const ExtPush pf = A.ext.ticks ? ext_push(A.ext, env, D.n) : ExtPush{};
+  ExtWrench<T> w;
+#pragma unroll
+  for (int i = 0; i < 3; i++) { w.f[i] = T(pf.w.f[i]); w.p[i] = T(pf.w.p[i]); }
   for (int t = 0; t < n_ticks; t++)
     {
     const EnvModelRef em{A.mass_randomizer ? D.model : nullptr, D.n, env};
-    if (physics_tick<T, true, 0, true>(st, t12, mu, cs, A.M, A.SC, true, scr, em, &A.M2)) { T dl[12]; physics_tick_general<T, true>(st, t12, mu, cs, A.M, A.SC, em, dl, 1); }
+    const ExtWrench<T>* ext = t < pf.n ? &w : nullptr;
+    if (physics_tick<T, true, 0, true, true>(st, t12, mu, cs, A.M, A.SC, true, scr, em, &A.M2, ext)) { T dl[12]; physics_tick_general<T, true, true>(st, t12, mu, cs, A.M, A.SC, em, dl, 1, ext); }
   }
+  if (pf.n > 0) A.ext.ticks[env] = pf.n - min(pf.n, n_ticks);
 #pragma unroll
   for (int i = 0; i < 3; i++) { sf.pos[i] = float(st.pos[i]); sf.vlin[i] = float(st.vlin[i]); sf.vang[i] = float(st.vang[i]); }
 #pragma unroll
@@ -142,6 +149,18 @@ k_debug_ticks(const __grid_constant__ DebugArgs<T> A, const float* __restrict__ 
   for (int i = 0; i < 12; i++) { sf.q[i] = float(st.q[i]); sf.qd[i] = float(st.qd[i]); }
   cf.mask = cs.mask; cf.invalid = cs.invalid;
   store_state(D, env, sf, cf, A.SC.dt);
+}
+
+// -------------------------------------------------------------------- push countdown (qs_set_external_force)
+// After a step of `consumed` ticks: n -= min(n, consumed), and n = 0 where `ended` is set (the step's done flags under
+// auto_reset: a push never carries into the next episode; the mask of a reset with consumed = 0).  ended == nullptr:
+// no env ended.  consumed < 0: every count goes to 0 (a reset of every env).
+__global__ void k_ext_countdown(int32_t* __restrict__ ticks, const uint8_t* __restrict__ ended, int consumed, int n) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= n) return;
+  const int32_t c = ticks[env];
+  if (consumed < 0 || (ended && ended[env])) { if (c != 0) ticks[env] = 0; }
+  else if (c > 0) ticks[env] = c - min(c, consumed);
 }
 
 // -------------------------------------------------------------------- K3: analytic utilities
@@ -356,6 +375,7 @@ struct qs_env {
   float* term_obs;     // caller-owned, optional (qs_set_terminal_obs)
   float* dev_demo;     // demonstration actions of the *_DEMO tasks (qs_set_demo)
   SubstepTrace trace;  // qs_set_substep_trace: caller-owned rows, column map in the pool (trace.buf == nullptr: off)
+  ExtForce ext;        // qs_set_external_force: caller-owned wrench and tick counts (ext.ticks == nullptr: off)
   bool was_reset;
   // CUDA-event ring around k_step launches (roofline timing of the dominant kernel)
   static constexpr int kRing = 512;
@@ -381,6 +401,13 @@ struct qs_env {
 };
 
 static inline unsigned grid_for(int n, int block) { return unsigned((n + block - 1) / block); }
+// f(em, trace, push) for every instantiation of the tick kernels, as std::bool_constant arguments
+template <typename F> static void for_each_tick_variant(F f) {
+  using T = std::true_type;
+  using N = std::false_type;
+  f(N{}, N{}, N{}); f(T{}, N{}, N{}); f(N{}, T{}, N{}); f(T{}, T{}, N{});
+  f(N{}, N{}, T{}); f(T{}, N{}, T{}); f(N{}, T{}, T{}); f(T{}, T{}, T{});
+}
 static int block_of(qs_handle) { return QS_BLOCK; }
 static size_t smem_of(int block) { return size_t(block) * QS_TICK_SCRATCH * sizeof(float); }
 
@@ -641,16 +668,15 @@ int qs_create(const qs_config* cfg, int n_envs, int device, qs_handle* out) {
   }
   {
     const int max_smem = int(smem_of(256));
-    e = cudaFuncSetAttribute(k_step<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    // the tick kernels' eight instantiations <mass randomizer, substep trace, push>
+    e = cudaSuccess;
+    for_each_tick_variant([&](auto em, auto trace, auto push) {
+      constexpr bool a = decltype(em)::value, b = decltype(trace)::value, c = decltype(push)::value;
+      if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step<a, b, c>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+      if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<a, b, c>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    });
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_reset<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_reset<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_step_contact<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_settle_urgent<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_settle_urgent<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_settle_slice<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
@@ -894,6 +920,11 @@ int qs_reset(qs_handle h, const uint8_t* mask, float* obs, void* stream) {
       if (int e = launch_slice(h, s, 0)) return e;
     }
   }
+  if (h->ext.ticks) {   // the reset envs' pushes end
+    k_ext_countdown<<<grid_for(h->n, 256), 256, 0, s>>>(h->ext.ticks, mask, mask ? 0 : -1, h->n);
+    g_launches += 1;
+    CUDA_TRY(cudaGetLastError());
+  }
   h->was_reset = true;
   return QS_OK;
 }
@@ -970,26 +1001,30 @@ static int step_impl(qs_handle h, const float* actions, float* obs, float* rewar
   io.stamps = h->stamps + 4 * slot;
   io.flight_cap = h->flight_cap;
   CUDA_TRY(rec_timing(h->ev0[slot], s, capturing));
-  // the tick kernels' instantiation: <mass randomizer, substep trace>
+  // the tick kernels' instantiation: <mass randomizer, substep trace, push>
   const SubstepTrace tr = h->trace;
+  const ExtForce ef = h->ext;
   auto tick_kernels = [&](auto launch) {
-    using T = std::true_type;
-    using F = std::false_type;
-    if (h->args.C.mass_randomizer) { if (tr.buf) launch(T{}, T{}); else launch(T{}, F{}); }
-    else { if (tr.buf) launch(F{}, T{}); else launch(F{}, F{}); }
+    for_each_tick_variant([&](auto em, auto trace, auto push) {
+      if (decltype(em)::value == bool(h->args.C.mass_randomizer) && decltype(trace)::value == (tr.buf != nullptr) &&
+          decltype(push)::value == (ef.ticks != nullptr))
+        launch(em, trace, push);
+    });
   };
   k_pre<<<grid_for(h->n, 256), 256, 0, s>>>(h->args, io);
   g_launches += 1;
-  tick_kernels([&](auto em, auto trace) {
-    k_step<decltype(em)::value, decltype(trace)::value><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io, tr);
+  tick_kernels([&](auto em, auto trace, auto push) {
+    k_step<decltype(em)::value, decltype(trace)::value, decltype(push)::value><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io,
+                                                                                                                   tr, ef);
   });
   if (h->cfg.auto_reset) {
     // conveyor, early slice: on the second stream, next to k_step_contact (about half a wave of blocks)
     if (int e = launch_conveyor(h, s, 0, 0)) return e;
     CUDA_TRY(cudaEventRecord(h->ev_fork0, s));
   }
-  tick_kernels([&](auto em, auto trace) {
-    k_step_contact<decltype(em)::value, decltype(trace)::value><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, io, tr);
+  tick_kernels([&](auto em, auto trace, auto push) {
+    k_step_contact<decltype(em)::value, decltype(trace)::value, decltype(push)::value><<<grid_for(h->n, B), B, smem_of(B), s>>>(
+        h->args, io, tr, ef);
   });
   g_launches += 1;
   // The epilogue of every env whose ticks are done (all but the general solver's).  With host buffers it runs here, so
@@ -1029,8 +1064,9 @@ static int step_impl(qs_handle h, const float* actions, float* obs, float* rewar
   // settle slice, which starts once every block of k_step_slow has been placed and runs next to it.  (Round 1 launched
   // the slice on a second stream: when the hardware placed it first, which it did on the three steps that follow a host
   // synchronisation, the general-solver blocks waited for the whole slice, +1 ms; a high-priority stream made it worse.)
-  tick_kernels([&](auto em, auto trace) {
-    k_step_slow<decltype(em)::value, decltype(trace)::value><<<grid_for(h->n, 64), 64, 0, s>>>(h->args, io, h->slow_spread, tr);
+  tick_kernels([&](auto em, auto trace, auto push) {
+    k_step_slow<decltype(em)::value, decltype(trace)::value, decltype(push)::value><<<grid_for(h->n, 64), 64, 0, s>>>(
+        h->args, io, h->slow_spread, tr, ef);
   });
   g_launches += 1;
   if (finish_late) {
@@ -1068,6 +1104,11 @@ static int step_impl(qs_handle h, const float* actions, float* obs, float* rewar
     if (h->args.C.mass_randomizer) k_settle_urgent<true><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, h->cv, obs); else k_settle_urgent<false><<<grid_for(h->n, B), B, smem_of(B), s>>>(h->args, h->cv, obs);
     k_urgent_clear<<<1, 1, 0, s>>>(h->cv);
     g_launches += 2;
+  }
+  if (ef.ticks) {
+    // the pushes' countdown, after every kernel that ran ticks of this step; ended episodes drop theirs
+    k_ext_countdown<<<grid_for(h->n, 256), 256, 0, s>>>(ef.ticks, h->cfg.auto_reset ? done : nullptr, h->args.C.action_repeat, h->n);
+    g_launches += 1;
   }
   CUDA_TRY(cudaGetLastError());
   h->launches_per_step = int(g_launches.load() - launches0);
@@ -1153,6 +1194,10 @@ int qs_reset_to_state(qs_handle h, const uint8_t* mask, const float* states, flo
   if (h->args.C.mass_randomizer) k_reset_state<true><<<grid_for(h->n, 128), 128, 0, s>>>(h->args, list, states, h->cv, obs);
   else k_reset_state<false><<<grid_for(h->n, 128), 128, 0, s>>>(h->args, list, states, h->cv, obs);
   g_launches += 1;
+  if (h->ext.ticks) {   // the reset envs' pushes end
+    k_ext_countdown<<<grid_for(h->n, 256), 256, 0, s>>>(h->ext.ticks, mask, mask ? 0 : -1, h->n);
+    g_launches += 1;
+  }
   CUDA_TRY(cudaGetLastError());
   if (!mask) h->was_reset = true;
   return QS_OK;
@@ -1196,6 +1241,17 @@ int qs_set_substep_trace(qs_handle h, const int32_t* env_ids, int n_traced, floa
   h->trace.buf = trace;
   h->trace.n_traced = trace ? n_traced : 0;
   drop_graphs(h);   // the trace is a kernel argument of the captured nodes
+  return QS_OK;
+}
+
+int qs_set_external_force(qs_handle h, float* wrench, int32_t* ticks) {
+  if (!h) return fail(QS_ERR_ARG, "handle is NULL");
+  if ((wrench == nullptr) != (ticks == nullptr)) return fail(QS_ERR_ARG, "wrench and ticks must both be set or both be NULL");
+  CUDA_TRY(cudaSetDevice(h->device));
+  CUDA_TRY(cudaDeviceSynchronize());  // no step may still be reading the old buffers
+  h->ext.wrench = wrench;
+  h->ext.ticks = ticks;
+  drop_graphs(h);   // the buffers are kernel arguments of the captured nodes, and the tick kernels change
   return QS_OK;
 }
 
@@ -1328,10 +1384,12 @@ int qs_debug_ticks(qs_handle h, const float* tau, int n_ticks, int use_f64, void
   if (use_f64) {
     DebugArgs<double> a;
     a.D = h->args.D; a.M = h->model_d; make_leg_pairs(a.M, a.M2); a.SC = h->args.SC; a.mass_randomizer = h->args.C.mass_randomizer;
+    a.ext = h->ext;
     k_debug_ticks<double><<<grid_for(h->n, 64), 64, 64 * QS_TICK_SCRATCH * sizeof(double), s>>>(a, tau, n_ticks);
   } else {
     DebugArgs<float> a;
     a.D = h->args.D; a.M = h->args.M; a.M2 = h->args.M2; a.SC = h->args.SC; a.mass_randomizer = h->args.C.mass_randomizer;
+    a.ext = h->ext;
     k_debug_ticks<float><<<grid_for(h->n, 64), 64, 64 * QS_TICK_SCRATCH * sizeof(float), s>>>(a, tau, n_ticks);
   }
   g_launches += 1;

@@ -241,6 +241,19 @@ QS_DEV void body_force(const SpI<T>& I, const T* Vw, const T* Vv, const T* Aw, c
 
 template <typename T> QS_DEV T clamp_vel(T v, T mx) { return fmin_t(fmax_t(v, T(-mx)), mx); }
 
+// External push on the base (Bullet applyExternalForce(robot, -1, f, pos + R p, WORLD_FRAME)): force f in the world frame
+// (N) at the point p, base frame, from the base origin (m).
+template <typename T> struct ExtWrench { T f[3]; T p[3]; };
+// The push as a spatial force in base coordinates about the base origin, (p x Rb^T f, Rb^T f), taken off the Newton-Euler
+// bias force fb: it acts on the body, the bias enters the base's equation with the opposite sign.
+template <typename T> QS_DEV void sub_ext_wrench(const T* Rb, const ExtWrench<T>& w, T* fb) {
+  T Fb[3], Nb[3];
+  m3t_v(Rb, w.f, Fb);
+  cross3(w.p, Fb, Nb);
+#pragma unroll
+  for (int i = 0; i < 3; i++) { fb[i] -= Nb[i]; fb[3 + i] -= Fb[i]; }
+}
+
 
 // ------------------------------------------------------------------------------------------
 // Shared pieces of a tick
@@ -639,14 +652,16 @@ template <typename T, typename ML> QS_DEV void leg_kin_from_sc(int k, const T* s
 enum { TICK_DONE = 0, TICK_NEEDS_GENERAL = 1, TICK_NEEDS_CONTACT = 2 };
 // kEM: read the per-env mass properties `em` (compiled out of the default kernels)
 // M2 != nullptr (float / double only): the per-leg passes run on PAIRS of legs with packed arithmetic (qs_packed.cuh).
+// kExt: `ext` != nullptr pushes the base in this tick (compiled out of the default kernels; a null `ext` runs the
+// arithmetic of the default instantiation).
 #ifndef QS_PACK_LEGS
 #define QS_PACK_LEGS 1
 #endif
-template <typename T, bool kContacts = true, int kStride = 0, bool kEM = false>
+template <typename T, bool kContacts = true, int kStride = 0, bool kEM = false, bool kExt = false>
 __host__ __device__ int physics_tick(EnvState<T>& st, const T* tau, T mu, ContactState<T>& cs,
                                      const ModelConstT<T>& M, const SolverConst& SC, bool detect_invalid,
                                      const Scratch<T, kStride>& scr, const EnvModelRef em = EnvModelRef{nullptr, 0, 0},
-                                     const ModelLegPairsT<T>* M2 = nullptr) {
+                                     const ModelLegPairsT<T>* M2 = nullptr, const ExtWrench<T>* ext = nullptr) {
   constexpr bool kPack = QS_PACK_LEGS && std::is_floating_point<T>::value;
   const T dt = T(SC.dt);
   const T idt = div_t(T(1), dt);
@@ -661,6 +676,9 @@ __host__ __device__ int physics_tick(EnvState<T>& st, const T* tau, T mu, Contac
   trunk_spi<T, kEM>(M, em, tot);
   T fb[6] = {T(0), T(0), T(0), T(0), T(0), T(0)};
   body_force(tot, X.wb, X.vb, zero3, X.A0, fb, fb + 3);
+  if constexpr (kExt) {
+    if (ext) sub_ext_wrench(X.Rb, *ext, fb);
+  }
   T S6[21];
 #pragma unroll
   for (int i = 0; i < 21; i++) S6[i] = T(0);
@@ -1281,10 +1299,12 @@ QS_DEV void body_point_jac(const LegKin<T>& K, int level, const T* pc, const T* 
   if (level < 1) Jk[1] = T(0);
 }
 
-template <typename T, bool kEM = false>
+// kExt / ext: as physics_tick
+template <typename T, bool kEM = false, bool kExt = false>
 __host__ __device__ void physics_tick_general(EnvState<T>& st, const T* tau, T mu, ContactState<T>& cs,
                                               const ModelConstT<T>& M, const SolverConst& SC,
-                                              const EnvModelRef em, T* dl /* 12 elements, stride dl_stride */, int dl_stride) {
+                                              const EnvModelRef em, T* dl /* 12 elements, stride dl_stride */, int dl_stride,
+                                              const ExtWrench<T>* ext = nullptr) {
   const T dt = T(SC.dt);
   const T mcv = T(SC.max_coord_vel);
   TickCtx<T> X;
@@ -1295,6 +1315,9 @@ __host__ __device__ void physics_tick_general(EnvState<T>& st, const T* tau, T m
   trunk_spi<T, kEM>(M, em, tot);
   T fb[6] = {T(0), T(0), T(0), T(0), T(0), T(0)};
   body_force(tot, X.wb, X.vb, zero3, X.A0, fb, fb + 3);
+  if constexpr (kExt) {
+    if (ext) sub_ext_wrench(X.Rb, *ext, fb);
+  }
   T S6[21];
   for (int i = 0; i < 21; i++) S6[i] = T(0);
   T Bm[4][18], ev[4][3], Mi[4][6];

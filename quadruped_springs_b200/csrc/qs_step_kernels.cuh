@@ -916,10 +916,10 @@ k_pre(const __grid_constant__ KernelArgs A, const StepIO io) {
 // The envs with no foot on the ground (dense warps: thread i takes flight_list[i]): flight variant of the tick, no
 // foot-contact code.  An env that reaches the ground goes on to k_step_contact as of the start of that tick.
 // kTrace (all three tick kernels): the variant launched while a substep trace is set (qs_set_substep_trace); `tr` is
-// read by that variant only
-template <bool kEM, bool kTrace>
+// read by that variant only.  kExt: likewise while a push buffer is attached (qs_set_external_force), `ef`.
+template <bool kEM, bool kTrace, bool kExt>
 __global__ void __launch_bounds__(256, 1)
-k_step(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace tr) {
+k_step(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace tr, const ExtForce ef) {
   const int tid = blockIdx.x * blockDim.x + threadIdx.x;
   const DeviceView& D = A.D;
   const EnvCfg& C = A.C;
@@ -943,8 +943,10 @@ k_step(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace
   extern __shared__ __align__(16) float qs_smem[];
   const StepScratch scr{qs_smem, QS_BLOCK, int(threadIdx.x)};
   int why;
-  const int t_done = run_ticks<false, kEM, kTrace>(st, cs, cmd, torque_mode, 0, C.action_repeat, env, D, C, A.RC, A.M, A.M2, A.SC, tau_m,
-                                              tau_s, true, scr, &why, kTrace ? trace_column(tr, env, live) : TraceColumn{nullptr, 0});
+  const int t_done = run_ticks<false, kEM, kTrace, kExt>(st, cs, cmd, torque_mode, 0, C.action_repeat, env, D, C, A.RC, A.M, A.M2, A.SC,
+                                                    tau_m, tau_s, true, scr, &why,
+                                                    kTrace ? trace_column(tr, env, live) : TraceColumn{nullptr, 0}, false,
+                                                    kExt ? ext_push(ef, env, n) : ExtPush{});
   if (!live) return;
   if (t_done < C.action_repeat) {
     park_env(A, io, env, st, cs, cmd, t_done, why == TICK_NEEDS_GENERAL ? io.slow_list : io.contact_list);
@@ -956,9 +958,9 @@ k_step(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace
 // -------------------------------------------------------------------- K1a: envs with foot contacts
 // Resumes the envs the flight kernel handed over (dense warps: thread i takes contact_list[i]) with
 // the full fast tick; joint limits / body contacts still go on to k_step_slow.
-template <bool kEM, bool kTrace>
+template <bool kEM, bool kTrace, bool kExt>
 __global__ void __launch_bounds__(256, 1)
-k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace tr) {
+k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io, const SubstepTrace tr, const ExtForce ef) {
   const int tid = blockIdx.x * blockDim.x + threadIdx.x;
   const DeviceView& D = A.D;
   const EnvCfg& C = A.C;
@@ -977,9 +979,10 @@ k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io, const Subs
   extern __shared__ __align__(16) float qs_smem[];
   const StepScratch scr{qs_smem, QS_BLOCK, int(threadIdx.x)};
   int why;
-  const int t_done = run_ticks<true, kEM, kTrace>(st, cs, cmd, torque_mode, D.resume_tick[env], C.action_repeat, env, D, C, A.RC, A.M,
-                                             A.M2, A.SC, tau_m, tau_s, true, scr, &why,
-                                             kTrace ? trace_column(tr, env, live) : TraceColumn{nullptr, 0});
+  const int t_done = run_ticks<true, kEM, kTrace, kExt>(st, cs, cmd, torque_mode, D.resume_tick[env], C.action_repeat, env, D, C, A.RC,
+                                                   A.M, A.M2, A.SC, tau_m, tau_s, true, scr, &why,
+                                                   kTrace ? trace_column(tr, env, live) : TraceColumn{nullptr, 0}, false,
+                                                   kExt ? ext_push(ef, env, n) : ExtPush{});
   if (!live) return;
   if (t_done < C.action_repeat) {
     park_env(A, io, env, st, cs, cmd, t_done, io.slow_list);
@@ -989,9 +992,9 @@ k_step_contact(const __grid_constant__ KernelArgs A, const StepIO io, const Subs
 }
 
 // -------------------------------------------------------------------- K1b: general-solver continuation
-template <bool kEM, bool kTrace>
+template <bool kEM, bool kTrace, bool kExt>
 __global__ void __launch_bounds__(64)
-k_step_slow(const __grid_constant__ KernelArgs A, const StepIO io, int spread, const SubstepTrace tr) {
+k_step_slow(const __grid_constant__ KernelArgs A, const StepIO io, int spread, const SubstepTrace tr, const ExtForce ef) {
   // Programmatic dependent launch: the late settle slice follows in the same stream and may start as soon as every block
   // of this grid has been placed (has got here or exited), not when the grid is complete.  That ordering is the point: the
   // slice fills every SM, and when the hardware happened to place it first (two streams racing), the few latency-bound
@@ -1021,9 +1024,16 @@ k_step_slow(const __grid_constant__ KernelArgs A, const StepIO io, int spread, c
   for (int i = 0; i < 12; i++) cmd[i] = D.cmd[i * n + env];
   const bool torque_mode = !A.C.is_rl && A.C.control_mode == QS_CTRL_TORQUE;
   __shared__ float dl_sm[12 * 64];   // the solver's per-leg vector delta (qs_physics.cuh GenRow), one column per thread
-  if constexpr (kTrace)
+  if constexpr (kTrace && kExt)
+    run_ticks_general<kEM, true, true>(st, cs, cmd, torque_mode, D.resume_tick[env], A.C.action_repeat, env, D, A.C, A.RC, A.M,
+                                       A.SC, tau_m, tau_s, dl_sm + threadIdx.x, 64, trace_column(tr, env, true),
+                                       ext_push(ef, env, n));
+  else if constexpr (kTrace)
     run_ticks_general<kEM, true>(st, cs, cmd, torque_mode, D.resume_tick[env], A.C.action_repeat, env, D, A.C, A.RC, A.M, A.SC,
                                  tau_m, tau_s, dl_sm + threadIdx.x, 64, trace_column(tr, env, true));
+  else if constexpr (kExt)
+    run_ticks_general<kEM, false, true>(st, cs, cmd, torque_mode, D.resume_tick[env], A.C.action_repeat, env, D, A.C, A.RC, A.M,
+                                        A.SC, tau_m, tau_s, dl_sm + threadIdx.x, 64, ext_push(ef, env, n));
   else
     run_ticks_general<kEM>(st, cs, cmd, torque_mode, D.resume_tick[env], A.C.action_repeat, env, D, A.C, A.RC, A.M, A.SC,
                       tau_m, tau_s, dl_sm + threadIdx.x, 64);

@@ -254,6 +254,83 @@ class BatchedQuadruped:
     def set_spring_rest_angles(self, rest):
         self._env._views["spring"][6:9] = torch.as_tensor(rest, dtype=torch.float32, device=self._env.device).view(3, -1)
 
+    # --- external push on the base (quadruped.py:338-343), applied tick by tick inside the step kernels
+    def apply_external_force(self, force, position=None, n_ticks=1, env_ids=None):
+        """Push the base of the envs `env_ids` (indices, a bool mask of [N], or None for every env) with `force` ([3] or
+        [k, 3], world frame, N) at `position` ([3] or [k, 3], base frame from GetBasePosition, m; default the base
+        position) for the next `n_ticks` physics ticks (int or [k] ints >= 0; a control step is action_repeat ticks).
+
+        In every tick it lasts, the push is Bullet's applyExternalForce(robot, -1, force, pos + R position, WORLD_FRAME)
+        made before that stepSimulation (qs_set_external_force has the full rule).  The count runs down by the ticks each
+        step runs; an episode end under auto_reset and a reset of the env set it to 0.  A call overwrites the selected
+        envs' force, point and count (n_ticks=0 cancels): unlike Bullet, where the calls made before one stepSimulation
+        add up.  The first call attaches the library's push buffers (clear_external_force detaches them)."""
+        env = self._env
+        dev, n = env.device, env.num_envs
+        if env_ids is None:
+            ids = torch.arange(n)
+        else:
+            ids = torch.as_tensor(env_ids).cpu()
+            if ids.dtype == torch.bool:
+                if ids.shape != (n,):
+                    raise ValueError(f"a bool env_ids mask must have shape ({n},), got {tuple(ids.shape)}")
+                ids = ids.nonzero().flatten()
+            elif ids.dtype in (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8) and ids.dim() <= 1:
+                ids = ids.reshape(-1).long()
+                if ids.numel() and (int(ids.min()) < 0 or int(ids.max()) >= n):
+                    raise ValueError(f"env_ids must lie in [0, {n})")
+                if ids.unique().numel() != ids.numel():
+                    raise ValueError("env_ids must be distinct")
+            else:
+                raise ValueError(f"env_ids must be indices or a bool mask, got {ids.dtype} of shape {tuple(ids.shape)}")
+        k = ids.numel()
+
+        def rows(x, name):
+            t = torch.as_tensor(x, dtype=torch.float64).cpu()
+            if t.shape == (3,):
+                t = t.expand(k, 3)
+            if t.shape != (k, 3):
+                raise ValueError(f"{name} must have shape (3,) or ({k}, 3), got {tuple(t.shape)}")
+            if not bool(torch.isfinite(t).all()):
+                raise ValueError(f"{name} must be finite")
+            return t.to(torch.float32)
+
+        f = rows(force, "force")
+        p = rows(torch.zeros(3) if position is None else position, "position")
+        nt = torch.as_tensor(n_ticks).cpu()
+        if nt.dtype.is_floating_point or nt.dtype == torch.bool or nt.dtype.is_complex:
+            raise ValueError(f"n_ticks must be integers, got {nt.dtype}")
+        if nt.dim() == 0:
+            nt = nt.expand(k)
+        if nt.shape != (k,):
+            raise ValueError(f"n_ticks must be an int or have shape ({k},), got {tuple(nt.shape)}")
+        if k and (int(nt.min()) < 0 or int(nt.max()) > 2**31 - 1):
+            raise ValueError("n_ticks must lie in [0, 2**31)")
+        if getattr(self, "_ext_ticks", None) is None:
+            wrench = torch.zeros(_lib.QS_EXT_DIM, n, device=dev)
+            ticks = torch.zeros(n, dtype=torch.int32, device=dev)
+            _lib.check(env._L.qs_set_external_force(env._h, _p(wrench), _p(ticks)))
+            self._ext_wrench, self._ext_ticks = wrench, ticks   # the library reads and counts them down: keep them alive
+        if k == 0:
+            return
+        ids = ids.to(dev)
+        self._ext_wrench[0:3, ids] = f.t().to(dev)
+        self._ext_wrench[3:6, ids] = p.t().to(dev)
+        self._ext_ticks[ids] = nt.to(device=dev, dtype=torch.int32)
+
+    def get_external_force(self):
+        """(force [N, 3], position [N, 3], ticks_left [N] int32): views of the attached push buffers (None when none is
+        attached).  ticks_left reads what the steps enqueued so far leave."""
+        if getattr(self, "_ext_ticks", None) is None:
+            return None
+        return self._ext_wrench[0:3].t(), self._ext_wrench[3:6].t(), self._ext_ticks
+
+    def clear_external_force(self):
+        """Detach the push buffers: every later step runs the kernels of an env that was never pushed."""
+        env = self._env
+        _lib.check(env._L.qs_set_external_force(env._h, None, None))
+        self._ext_wrench = self._ext_ticks = None
+
 
 class _ActionInterface:
     """control_interface/interface_base.py + motor_interface.py on batches."""
