@@ -1230,7 +1230,7 @@ __host__ __device__ int physics_tick(EnvState<T>& st, const T* tau, T mu, Contac
 // link order (trunk, imu, then hip/thigh/calf/foot per leg), all friction cones.
 // Rows live in local memory: this runs for the handful of envs the fast tick hands over.
 // ------------------------------------------------------------------------------------------
-constexpr int QS_MAX_CONTACTS = 17;
+constexpr int QS_MAX_CONTACTS = 2 + 4 * 4;   // every shape can touch at once: trunk, imu, and hip, thigh, calf, foot per leg
 constexpr int QS_MAX_LIMITS = 12;
 
 // A general row over u = [z(6), delta_leg0(3), ..., delta_leg3(3)]:  w = a . u,  u += b dI  with a = [Y, Jk in the
