@@ -357,6 +357,26 @@ int qs_set_substep_trace(qs_handle h, const int32_t* env_ids_dev, int n_traced, 
 #define QS_EXT_DIM 6   /* rows: force xyz (world, N), point xyz (base frame, from the base position, m) */
 int qs_set_external_force(qs_handle h, float* wrench_dev /*[QS_EXT_DIM][N]*/, int32_t* ticks_dev /*[N]*/);
 
+/* Camera images of robots (QuadrupedGymEnv.render(mode="rgb_array") -> pybullet getCameraImage,
+ * quadruped_gym_env.py render; utils/video_recording.py): image i shows the robot of states_dev row i (qs_get_state
+ * rows, so recorded states render as well) on the ground plane, seen by camera row i = pybullet's view matrix (16) then
+ * projection matrix (16), column-major as computeViewMatrix* / computeProjectionMatrix* return them.  Stateless, needs
+ * no handle.  Drawn: the plane z = 0 (1 m checkerboard) and the 18 collision primitives the contact code collides (the
+ * mass randomizer's payload block is not drawn), one flat colour per link kind, one directional light with shadows of
+ * the robot.  Pixel (r, c), row 0 at the top, is the ray through its centre, x_ndc = 2 (c + 0.5) / W - 1,
+ * y_ndc = 1 - 2 (r + 0.5) / H, unprojected through inverse(P V) from the near to the far plane; no anti-aliasing.
+ *   rgb_dev   [k][H][W][3] uint8, sky colour for a miss
+ *   depth_dev [k][H][W] metric eye-space depth -z_eye (pybullet's depth buffer d linearised as
+ *             far near / (far - (far - near) d)); far for a miss
+ *   seg_dev   [k][H][W] ER_SEGMENTATION_MASK_OBJECT_AND_LINKINDEX: objectUniqueId + ((linkIndex + 1) << 24), plane 0
+ *             (object 0, link -1), robot object 1 with URDF link indices (trunk 0, imu 1, then hip, thigh, calf, foot of
+ *             FR, FL, RR, RL: feet 5, 9, 13, 17); -1 for a miss
+ * Any of the three may be NULL, not all.  A state row with a non-finite word draws no robot.  QS_ERR_ARG when k < 1,
+ * width or height is outside [1, 4096], or no output is given.  Launches one kernel on `stream`. */
+#define QS_CAM_DIM 32
+int qs_render(const float* states_dev /*[k, QS_STATE_DIM]*/, const float* cams_dev /*[k, QS_CAM_DIM]*/, int k, int width,
+              int height, uint8_t* rgb_dev, float* depth_dev, int32_t* seg_dev, void* stream);
+
 /* number of kernels launched by this library since load (bench bookkeeping) */
 int64_t qs_launch_count(void);
 

@@ -5,9 +5,10 @@ from .env import (  # noqa: F401
     MotorInterfaceCollection, SensorCollection, TaskCollection,
 )
 from .hopf_network import HopfNetwork  # noqa: F401
-from . import demo, load_model, ops, stats, substep, vec_env  # noqa: F401
+from . import demo, load_model, ops, render, stats, substep, vec_env  # noqa: F401
+from .render import VideoRecorder  # noqa: F401
 from .substep import SubstepRecorder  # noqa: F401
 from .vec_env import BatchedVecEnv, MlpPolicyTorch, VecNormalizeTorch  # noqa: F401
 
 __all__ = ["BatchedQuadrupedGymEnv", "BatchedQuadruped", "HopfNetwork", "ops", "BatchedVecEnv", "VecNormalizeTorch",
-           "MlpPolicyTorch", "SubstepRecorder"]
+           "MlpPolicyTorch", "SubstepRecorder", "VideoRecorder", "render"]

@@ -10,7 +10,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libqs_b200.so")
-SOURCES = ["qs_kernels.cu", "qs_step_kernels.cuh", "qs_env.cuh", "qs_physics.cuh", "qs_packed.cuh", "qs_robot.cuh", "qs_types.h", "qs_model_host.h"]
+SOURCES = ["qs_kernels.cu", "qs_render.cu", "qs_step_kernels.cuh", "qs_env.cuh", "qs_physics.cuh", "qs_packed.cuh", "qs_robot.cuh", "qs_types.h", "qs_model_host.h"]
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "qs_b200.h")
 
 NVCC_FLAGS = [
@@ -24,6 +24,7 @@ QS_STATS_DIM = 16
 QS_STATE_DIM = 37
 QS_TRACE_DIM = 66   # row of the per-substep trace (qs_set_substep_trace)
 QS_EXT_DIM = 6      # rows of the push wrench (qs_set_external_force): force xyz (world, N), point xyz (base frame, m)
+QS_CAM_DIM = 32     # camera row of qs_render: view matrix (16) then projection matrix (16), column-major
 
 
 class QsConfig(C.Structure):
@@ -81,7 +82,7 @@ def build(force=False, verbose=False):
                 return SO_PATH
             tmp = f"{SO_PATH}.{os.getpid()}.tmp"
             cmd = [nvcc_path()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + [
-                "-o", tmp, os.path.join(CSRC, "qs_kernels.cu")]
+                "-o", tmp] + [os.path.join(CSRC, s) for s in SOURCES if s.endswith(".cu")]
             res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
             if res.returncode != 0:
                 if os.path.exists(tmp):
@@ -141,6 +142,8 @@ EXPORTS = {
     "qs_slow_kernel_time": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_float)]),
     "qs_step_count": (C.c_int64, [C.c_void_p]),
     "qs_timing_window": (C.c_int, [C.c_void_p]),
+    "qs_render": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                            C.c_void_p]),
     "qs_launch_count": (C.c_int64, []),
 }
 

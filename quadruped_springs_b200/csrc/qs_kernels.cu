@@ -40,6 +40,11 @@ static int fail(int code, const std::string& msg) {
   g_err = msg;
   return code;
 }
+// the library's other translation unit (qs_render.cu) reports errors and counts launches through these
+namespace qs {
+int abi_fail(int code, const std::string& msg) { return fail(code, msg); }
+void abi_count_launch() { g_launches += 1; }
+}  // namespace qs
 #define CUDA_TRY(expr)                                                                       \
   do {                                                                                       \
     cudaError_t _e = (expr);                                                                 \

@@ -528,7 +528,8 @@ class BatchedQuadrupedGymEnv:
         jumped, stands on its four feet and its base rises again, the env ramps to the init action on gains 60 / 0.8
         (60 / 1.5 without springs) until the episode ends (infos["rest_active"])."""
         if render or on_rack:
-            raise ValueError("render / on_rack are visual-debug modes of the pybullet GUI and are not provided")
+            raise ValueError("render=True (the pybullet GUI) and on_rack are not provided; camera images come from "
+                             "env.render('rgb_array') and env.render_images()")
         self._L = _lib.lib()
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedQuadrupedGymEnv needs a CUDA device; there is no CPU fallback")
@@ -782,6 +783,26 @@ class BatchedQuadrupedGymEnv:
         t = torch.as_tensor(tau, dtype=torch.float32, device=self.device).contiguous()
         assert t.shape == (self.num_envs, 12)
         _lib.check(self._L.qs_debug_ticks(self._h, _p(t), int(n_ticks), int(use_f64), _stream_ptr(self.device)))
+
+    # ------------------------------------------------------------------ camera images (quadruped_springs_b200/render.py)
+    def render(self, mode="rgb_array"):
+        """QuadrupedGymEnv.render: env 0's image of the follow camera as a numpy uint8 [360, 480, 3] for "rgb_array",
+        an empty array for any other mode (there is no GUI)."""
+        if mode != "rgb_array":
+            return np.array([])
+        return self.render_images([0])["rgb"][0].cpu().numpy()
+
+    def render_images(self, env_ids=None, width=480, height=360, camera=None, depth=False, segmentation=False):
+        """Camera images of the envs `env_ids` (all when None) in their current state: render.render_states of
+        get_state()[env_ids] through `camera` ([k, 32] or [32], pybullet's view then projection matrix) or, by default,
+        the follow camera of each robot.  Returns a dict of CUDA tensors ("rgb", and "depth" / "segmentation" when
+        asked).  Reads the state only: no env value changes."""
+        from .render import follow_cameras, render_states
+        states = self.get_state()
+        if env_ids is not None:
+            states = states[torch.as_tensor(env_ids, dtype=torch.long, device=self.device)]
+        cams = camera if camera is not None else follow_cameras(states[:, :3], width, height)
+        return render_states(states, cams, width, height, rgb=True, depth=depth, segmentation=segmentation)
 
     # ------------------------------------------------------------------ getters (quadruped_gym_env.py:343-426)
     def get_observation(self, with_noise=True):

@@ -25,6 +25,7 @@ import numpy as np
 import torch
 
 from .env import BatchedQuadrupedGymEnv
+from .render import tile_images
 
 
 class BatchedVecEnv:
@@ -32,9 +33,10 @@ class BatchedVecEnv:
     BatchedQuadrupedGymEnv.  `callable_env` of load_model.py:88-99 maps to kwargs: `go_to_rest_wrapper=True`,
     `landing_wrapper="LandingWrapper2"`, ...; the observation is already flat (ObsFlatteningWrapper)."""
 
-    metadata = {"render.modes": []}
+    metadata = {"render.modes": ["rgb_array"]}
 
-    def __init__(self, env=None, num_envs=None, device="cuda", **env_kwargs):
+    def __init__(self, env=None, num_envs=None, device="cuda", render_env_ids=(0,), **env_kwargs):
+        """render_env_ids: the envs whose follow-camera images get_images() / render() return."""
         if env is None:
             env = BatchedQuadrupedGymEnv(num_envs=num_envs, device=device, auto_reset=True, **env_kwargs)
         if not env._auto_reset:
@@ -44,6 +46,9 @@ class BatchedVecEnv:
         self.observation_space = env.observation_space
         self.action_space = env.action_space
         self.device = env.device
+        self.render_env_ids = [int(i) for i in render_env_ids]
+        if not self.render_env_ids or not all(0 <= i < env.num_envs for i in self.render_env_ids):
+            raise ValueError(f"render_env_ids must be a non-empty list of env indices in [0, {env.num_envs})")
         n, o = env.num_envs, env.obs_dim
         self._term_obs = torch.zeros(n, o, device=env.device)
         env.set_terminal_obs_buffer(self._term_obs)
@@ -129,10 +134,15 @@ class BatchedVecEnv:
         return [False for _ in self._indices(indices)]
 
     def get_images(self):
-        raise NotImplementedError("rendering is out of scope (DESIGN.md section 7)")
+        """One follow-camera image (numpy uint8 [360, 480, 3]) per env of render_env_ids (VecVideoRecorder's source)."""
+        return list(self.env.render_images(self.render_env_ids)["rgb"].cpu().numpy())
 
-    def render(self, mode="human"):
-        raise NotImplementedError("rendering is out of scope (DESIGN.md section 7)")
+    def render(self, mode="rgb_array"):
+        """The images of get_images() tiled as stable-baselines3's VecEnv.render does (render.tile_images).  There is
+        no GUI, so "rgb_array" is the only mode."""
+        if mode != "rgb_array":
+            raise NotImplementedError(f"render mode {mode!r} needs a GUI; only 'rgb_array' is provided")
+        return tile_images(self.get_images())
 
     @property
     def unwrapped(self):
