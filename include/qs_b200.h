@@ -377,6 +377,54 @@ int qs_set_external_force(qs_handle h, float* wrench_dev /*[QS_EXT_DIM][N]*/, in
 int qs_render(const float* states_dev /*[k, QS_STATE_DIM]*/, const float* cams_dev /*[k, QS_CAM_DIM]*/, int k, int width,
               int height, uint8_t* rgb_dev, float* depth_dev, int32_t* seg_dev, void* stream);
 
+/* ---- ARS training (sb3_contrib.ars.ARS with one candidate policy per group of envs; quadruped_springs_b200/ars.py) ----
+ * Two stateless entry points, run once per control step beside qs_step.  Neither synchronises the host. */
+
+/* Running observation statistics (VecNormalize.obs_rms, RunningMeanStd.update, float64) and episode bookkeeping.
+ * Statistics (mean_dev, var_dev, count_dev all non-NULL): the rows r of obs_dev [n, o] with alive_dev[r] != 0 (every row
+ * when alive_dev is NULL) form one batch; its mean and population variance are merged into the running mean, var and
+ * count (Chan et al.) exactly as RunningMeanStd.update merges them.  No alive row leaves all three unchanged.  count_dev
+ * lives on the device because the host does not know how many rows are alive.  mean_dev == NULL skips the statistics
+ * (obs_dev may then be NULL).
+ * Bookkeeping (reward_dev, done_dev, ret_dev, len_dev all non-NULL; alive_dev required): for every row r,
+ *   if alive[r]: ret[r] += reward[r] (float64), len[r] += 1;  then alive[r] &= !done[r]
+ * after the row has been read for the statistics, so the statistics of a step see the envs that were alive before it.
+ * QS_ERR_ARG when n < 1, o is outside [1, QS_MAX_OBS] (with statistics), or neither part is requested.  One launch of
+ * one 8-block cluster: the result does not depend on the launch, only on the rows and their order. */
+int qs_obs_stats(const float* obs_dev /*[n, o]*/, uint8_t* alive_dev /*[n] or NULL*/, int n, int o, double* mean_dev,
+                 double* var_dev, double* count_dev /*[1]*/, const float* reward_dev, const uint8_t* done_dev,
+                 double* ret_dev, int32_t* len_dev, void* stream);
+
+/* The policy network of sb3-contrib's ARSPolicy / ARSLinearPolicy: Linear layers (weight [out, in] row-major, then bias
+ * when `bias`), `activation` after each hidden layer, tanh on the output when `squash`. */
+#define QS_ARS_MAX_HIDDEN 64
+#define QS_ARS_MAX_ACT 12
+#define QS_ARS_RELU 0
+#define QS_ARS_TANH 1
+typedef struct {
+  int32_t obs_dim;      /* [1, QS_MAX_OBS] */
+  int32_t act_dim;      /* [1, QS_ARS_MAX_ACT] */
+  int32_t n_hidden;     /* 0, 1 or 2 */
+  int32_t hidden[2];    /* each in [1, QS_ARS_MAX_HIDDEN] (the first n_hidden) */
+  int32_t activation;   /* QS_ARS_RELU or QS_ARS_TANH */
+  int32_t bias;         /* 0 or 1 */
+  int32_t squash;       /* 0 or 1 */
+} qs_ars_arch;
+
+/* Actions of ARS candidate policies.  Env e (row e of obs_dev) runs candidate c = first_candidate + e / envs_per_candidate,
+ * whose parameter vector is theta + delta_std * deltas[c] for c < n_delta and theta - delta_std * deltas[c - n_delta]
+ * otherwise (each product rounded to fp32 before the sum, as torch computes it); deltas_dev == NULL means theta itself
+ * for every env.  theta [P] is parameters_to_vector of the policy (layer by layer: weight row-major, then bias).  The
+ * observation is first normalised as VecNormalize does, in float64: clip((obs - mean) / sqrt(var + eps), +-clip_obs),
+ * rounded to fp32 (mean_dev == NULL: no normalisation).  Output actions_dev [n, act_dim], clipped to [-1, 1].
+ * A block evaluates envs of one candidate, forming that candidate's weights once into shared memory; an env's action
+ * does not depend on the other envs of the call.  QS_ERR_ARG for an arch outside the ranges above, n < 1,
+ * envs_per_candidate < 1, n_delta < 1, or a candidate index outside [0, 2 n_delta).  One launch. */
+int qs_ars_act(const float* obs_dev /*[n, obs_dim]*/, const double* mean_dev, const double* var_dev, double clip_obs,
+               double eps, const float* theta_dev /*[P]*/, const float* deltas_dev /*[n_delta, P] or NULL*/,
+               float delta_std, int n_delta, int first_candidate, int envs_per_candidate, const qs_ars_arch* arch,
+               float* actions_dev /*[n, act_dim]*/, int n, void* stream);
+
 /* number of kernels launched by this library since load (bench bookkeeping) */
 int64_t qs_launch_count(void);
 

@@ -10,7 +10,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libqs_b200.so")
-SOURCES = ["qs_kernels.cu", "qs_render.cu", "qs_step_kernels.cuh", "qs_env.cuh", "qs_physics.cuh", "qs_packed.cuh", "qs_robot.cuh", "qs_types.h", "qs_model_host.h"]
+SOURCES = ["qs_kernels.cu", "qs_render.cu", "qs_ars.cu", "qs_step_kernels.cuh", "qs_env.cuh", "qs_physics.cuh", "qs_packed.cuh", "qs_robot.cuh", "qs_types.h", "qs_model_host.h"]
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "qs_b200.h")
 
 NVCC_FLAGS = [
@@ -25,6 +25,9 @@ QS_STATE_DIM = 37
 QS_TRACE_DIM = 66   # row of the per-substep trace (qs_set_substep_trace)
 QS_EXT_DIM = 6      # rows of the push wrench (qs_set_external_force): force xyz (world, N), point xyz (base frame, m)
 QS_CAM_DIM = 32     # camera row of qs_render: view matrix (16) then projection matrix (16), column-major
+QS_ARS_MAX_HIDDEN = 64
+QS_ARS_MAX_ACT = 12
+QS_ARS_RELU, QS_ARS_TANH = 0, 1
 
 
 class QsConfig(C.Structure):
@@ -45,6 +48,12 @@ class QsConfig(C.Structure):
         ("rand_payload_max", C.c_float), ("rand_payload_pos", C.c_float * 3), ("rand_spring_err", C.c_float),
         ("self_collision", C.c_int32),
     ]
+
+
+class QsArsArch(C.Structure):
+    """qs_ars_arch: the network of sb3-contrib's ARSPolicy / ARSLinearPolicy that qs_ars_act evaluates"""
+    _fields_ = [("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("n_hidden", C.c_int32), ("hidden", C.c_int32 * 2),
+                ("activation", C.c_int32), ("bias", C.c_int32), ("squash", C.c_int32)]
 
 
 class QsStatePtrs(C.Structure):
@@ -144,6 +153,9 @@ EXPORTS = {
     "qs_timing_window": (C.c_int, [C.c_void_p]),
     "qs_render": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                             C.c_void_p]),
+    "qs_obs_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 8),
+    "qs_ars_act": (C.c_int, [C.c_void_p] * 3 + [C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_float, C.c_int,
+                             C.c_int, C.c_int, C.POINTER(QsArsArch), C.c_void_p, C.c_int, C.c_void_p]),
     "qs_launch_count": (C.c_int64, []),
 }
 

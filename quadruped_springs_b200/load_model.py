@@ -63,16 +63,22 @@ def adapt_args(kwargs):
         kwargs.pop(e, None)
 
 
+def replay_env_kwargs(training_kwargs, task, render=False):
+    """load_model.py:79-85: training kwargs -> the kwargs of the replay env (ground randomizer, the given task)"""
+    env_kwargs = dict(training_kwargs)
+    env_kwargs["render"] = render
+    env_kwargs["env_randomizer_mode"] = "GROUND_RANDOMIZER"
+    env_kwargs["task_env"] = task
+    adapt_args(env_kwargs)
+    return env_kwargs
+
+
 def get_env_kwargs(src, task, render=False, env_name=ENV_NAME):
     """load_model.py:77-85: the training kwargs with the task / randomizer the replay wants"""
     env_kwargs = {}
     loaded_args = load_env_kwargs(src, env_name)
     if loaded_args.get("env_kwargs") is not None:
-        env_kwargs = dict(loaded_args["env_kwargs"])
-        env_kwargs["render"] = render
-        env_kwargs["env_randomizer_mode"] = "GROUND_RANDOMIZER"
-        env_kwargs["task_env"] = task
-        adapt_args(env_kwargs)
+        env_kwargs = replay_env_kwargs(loaded_args["env_kwargs"], task, render)
     return env_kwargs
 
 
@@ -227,14 +233,21 @@ def replay(source_path, task, algo="ppo", model="best_model.zip", n_envs=1, devi
     venv = make_vec_env(env_kwargs, n_envs=n_envs, device=device, **make_kwargs)
     vn = load_vecnormalize(os.path.join(source_path, ENV_NAME, "vecnormalize.pkl"), venv)
     policy = load_policy(os.path.join(source_path, model), algo, device)
+    ret = first_episode_returns(vn, policy, max_steps)
+    venv.close()
+    return ret
+
+
+def first_episode_returns(vn, policy, max_steps=1500):
+    """`model.predict(obs, deterministic=True)` on the normalised env until every env has finished its first episode
+    (load_model.py:126-134): the undiscounted return of that episode per env [num_envs] (numpy)"""
     obs = vn.reset()
-    ret = torch.zeros(n_envs, device=device)
-    alive = torch.ones(n_envs, dtype=torch.bool, device=device)
+    ret = torch.zeros(vn.num_envs, device=obs.device)
+    alive = torch.ones(vn.num_envs, dtype=torch.bool, device=obs.device)
     for _ in range(max_steps):
         obs, reward, done, _ = vn.step(policy.predict(obs, deterministic=True))
         ret += torch.where(alive, vn.get_original_reward(), torch.zeros_like(ret))
         alive &= ~done
         if not bool(alive.any()):
             break
-    venv.close()
     return ret.cpu().numpy()
