@@ -425,6 +425,91 @@ int qs_ars_act(const float* obs_dev /*[n, obs_dim]*/, const double* mean_dev, co
                float delta_std, int n_delta, int first_candidate, int envs_per_candidate, const qs_ars_arch* arch,
                float* actions_dev /*[n, act_dim]*/, int n, void* stream);
 
+/* ---- PPO training (stable_baselines3.PPO with VecNormalize over the batch; quadruped_springs_b200/ppo.py) ----
+ * Three stateless entry points.  Per control step qs_ppo_act runs before qs_step, qs_obs_stats (statistics only) and
+ * qs_ppo_reward after it; qs_ppo_gae runs once per rollout.  None synchronises the host.  Rollout buffers are step-major:
+ * row t of a [n_steps, n, ...] array holds step t of every env. */
+
+/* The network of SB3's ActorCriticPolicy with the default MlpExtractor and one net_arch for both heads.  theta is
+ * parameters_to_vector of MlpPolicyTorch, in this order (torch lists a module's own parameters before its children's;
+ * each Linear: weight [out, in] row-major, then bias [out]):
+ *   log_std                   [act_dim]
+ *   mlp_extractor.policy_net  n_hidden Linear layers (obs_dim -> hidden[0] -> hidden[1])
+ *   mlp_extractor.value_net   the same shapes
+ *   action_net                Linear(last, act_dim), last = hidden[n_hidden - 1] or obs_dim
+ *   value_net                 Linear(last, 1)
+ * `activation` follows every hidden layer. */
+typedef struct {
+  int32_t obs_dim;      /* [1, QS_MAX_OBS] */
+  int32_t act_dim;      /* [1, QS_ARS_MAX_ACT] */
+  int32_t n_hidden;     /* 0, 1 or 2 */
+  int32_t hidden[2];    /* each in [1, QS_ARS_MAX_HIDDEN] (the first n_hidden) */
+  int32_t activation;   /* QS_ARS_RELU or QS_ARS_TANH */
+} qs_ppo_arch;
+
+/* Pointers and scalars of one qs_ppo_act call (device pointers; NULL where a field is not used). */
+typedef struct {
+  const float* obs;                /* [n, obs_dim] raw observations of step `step` */
+  const double* obs_mean;          /* [obs_dim] running statistics (VecNormalize.obs_rms); NULL: no normalisation */
+  const double* obs_var;           /* [obs_dim] */
+  const float* theta;              /* [P], see qs_ppo_arch */
+  const uint8_t* episode_start;    /* [n] 1 where step `step` starts an episode (the previous step's done) */
+  const uint8_t* prev_truncated;   /* [n] the previous step's TimeLimit.truncated; NULL: no bootstrap */
+  const float* terminal_obs;       /* [n, obs_dim] raw terminal observations of the previous step (qs_set_terminal_obs) */
+  float* actions;                  /* [n, act_dim] the env action: the sample (or the mean) clipped to [-1, 1] */
+  float* buf_obs;                  /* [n_steps, n, obs_dim] normalised observations */
+  float* buf_actions;              /* [n_steps, n, act_dim] unclipped samples */
+  float* buf_values;               /* [n_steps, n] */
+  float* buf_log_probs;            /* [n_steps, n] */
+  float* buf_episode_starts;       /* [n_steps, n] 0 / 1 */
+  float* buf_rewards;              /* [n_steps, n] the bootstrap adds to row step - 1 */
+  float* last_values;              /* [n] values_only: V of the observations */
+  float* mean_out;                 /* [n, act_dim] or NULL: the actor mean */
+  double clip_obs, epsilon;        /* VecNormalize's clip_obs and epsilon */
+  uint64_t seed;                   /* key of the policy noise */
+  int64_t env_id_offset;           /* global id of row 0 (shards) */
+  float gamma;                     /* discount of the bootstrap */
+  int32_t iteration;               /* rollout index: part of the noise key */
+  int32_t step;                    /* in [0, n_steps) for a sampling call, in [0, n_steps] otherwise */
+  int32_t n_steps;
+  int32_t n;
+  int32_t values_only;             /* 1: last_values and the bootstrap only */
+  int32_t deterministic;           /* 1: actions = clipped mean, nothing else is written (but mean_out) */
+} qs_ppo_args;
+
+/* Actor and critic of every env (one thread per env).  The observation is normalised as VecNormalize does, in float64:
+ * clip((obs - mean) / sqrt(var + eps), +-clip_obs), rounded to fp32 (the same bits as VecNormalizeTorch.normalize_obs).
+ * A sampling call draws eps ~ N(0, 1) per action entry from Philox keyed by (seed, env_id_offset + row, iteration, step),
+ * a = mean + exp(log_std) eps, log_prob = sum_i log N(a_i; mean_i, std_i), and writes row `step` of every buffer
+ * (normalised obs, a, V, log_prob, episode start) and the clipped env action.  Where episode_start and prev_truncated
+ * are both set, buf_rewards[step - 1] += gamma V(normalised terminal_obs), SB3's time-limit bootstrap; the terminal
+ * observation is normalised with the same statistics as the step's own.  values_only writes last_values and that
+ * bootstrap (call it with step = n_steps after the last step).  QS_ERR_ARG for an arch outside its ranges, n < 1, a
+ * step outside [0, n_steps) for a sampling call or outside [0, n_steps] for the others, or a missing pointer the call
+ * needs.  One launch. */
+int qs_ppo_act(const qs_ppo_args* args, const qs_ppo_arch* arch, void* stream);
+
+/* VecNormalize's reward path and Monitor's episode totals for one step of n envs (one 8-block cluster):
+ *   ret = ret * gamma + reward (float64); every row's ret merged into ret_rms (mean, var, count [1] each; Chan et al. in
+ *   a fixed order, then RunningMeanStd.update_from_moments); reward_out = clip(reward / sqrt(var + epsilon),
+ *   +-clip_reward) with the updated var, rounded to fp32; ret = 0 where done.
+ *   ep_return += reward (float64), ep_length += 1; where done they are added to totals[0..2] = {episodes, sum of returns,
+ *   sum of lengths} and cleared; totals[3] += the sum of every row's reward (fixed order; totals [4] may be NULL).
+ * ret, ret_mean, ret_var and ret_count all NULL: no normalisation, reward_out = reward.  The result does not depend on
+ * the launch, only on the rows and their order. */
+int qs_ppo_reward(const float* reward_dev, const uint8_t* done_dev, int n, double* ret_dev, double* ret_mean_dev,
+                  double* ret_var_dev, double* ret_count_dev, double gamma, double epsilon, double clip_reward,
+                  float* reward_out_dev, double* ep_return_dev, int32_t* ep_length_dev, double* totals_dev,
+                  void* stream);
+
+/* RolloutBuffer.compute_returns_and_advantage over step-major [n_steps, n] arrays, fp32 operation for operation:
+ * next_non_terminal = 1 - last_dones (last step) or 1 - episode_starts[t + 1], next_values = last_values or
+ * values[t + 1], delta = rewards[t] + gamma next_values next_non_terminal - values[t],
+ * adv[t] = delta + gamma gae_lambda next_non_terminal adv[t + 1]; returns = adv + values.  One launch. */
+int qs_ppo_gae(const float* rewards_dev, const float* values_dev, const float* episode_starts_dev,
+               const float* last_values_dev /*[n]*/, const uint8_t* last_dones_dev /*[n]*/, int n_steps, int n,
+               double gamma, double gae_lambda, float* advantages_dev, float* returns_dev, void* stream);
+
 /* number of kernels launched by this library since load (bench bookkeeping) */
 int64_t qs_launch_count(void);
 

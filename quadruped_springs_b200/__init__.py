@@ -5,11 +5,12 @@ from .env import (  # noqa: F401
     MotorInterfaceCollection, SensorCollection, TaskCollection,
 )
 from .ars import BatchedARS  # noqa: F401
+from .ppo import BatchedPPO  # noqa: F401
 from .hopf_network import HopfNetwork  # noqa: F401
-from . import ars, demo, load_model, ops, render, stats, substep, vec_env  # noqa: F401
+from . import ars, demo, load_model, ops, ppo, render, stats, substep, vec_env  # noqa: F401
 from .render import VideoRecorder  # noqa: F401
 from .substep import SubstepRecorder  # noqa: F401
 from .vec_env import BatchedVecEnv, MlpPolicyTorch, VecNormalizeTorch  # noqa: F401
 
 __all__ = ["BatchedQuadrupedGymEnv", "BatchedQuadruped", "HopfNetwork", "ops", "BatchedVecEnv", "VecNormalizeTorch",
-           "MlpPolicyTorch", "SubstepRecorder", "VideoRecorder", "render", "BatchedARS"]
+           "MlpPolicyTorch", "SubstepRecorder", "VideoRecorder", "render", "BatchedARS", "BatchedPPO"]

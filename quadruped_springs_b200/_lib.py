@@ -10,7 +10,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libqs_b200.so")
-SOURCES = ["qs_kernels.cu", "qs_render.cu", "qs_ars.cu", "qs_step_kernels.cuh", "qs_env.cuh", "qs_physics.cuh", "qs_packed.cuh", "qs_robot.cuh", "qs_types.h", "qs_model_host.h"]
+SOURCES = ["qs_kernels.cu", "qs_render.cu", "qs_ars.cu", "qs_ppo.cu", "qs_step_kernels.cuh", "qs_env.cuh", "qs_physics.cuh", "qs_packed.cuh", "qs_robot.cuh", "qs_types.h", "qs_model_host.h"]
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "qs_b200.h")
 
 NVCC_FLAGS = [
@@ -54,6 +54,22 @@ class QsArsArch(C.Structure):
     """qs_ars_arch: the network of sb3-contrib's ARSPolicy / ARSLinearPolicy that qs_ars_act evaluates"""
     _fields_ = [("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("n_hidden", C.c_int32), ("hidden", C.c_int32 * 2),
                 ("activation", C.c_int32), ("bias", C.c_int32), ("squash", C.c_int32)]
+
+
+class QsPpoArch(C.Structure):
+    """qs_ppo_arch: the actor-critic network of SB3's ActorCriticPolicy that qs_ppo_act evaluates"""
+    _fields_ = [("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("n_hidden", C.c_int32), ("hidden", C.c_int32 * 2),
+                ("activation", C.c_int32)]
+
+
+class QsPpoArgs(C.Structure):
+    """qs_ppo_args: the pointers and scalars of one qs_ppo_act call"""
+    _fields_ = [(n, C.c_void_p) for n in (
+        "obs", "obs_mean", "obs_var", "theta", "episode_start", "prev_truncated", "terminal_obs", "actions", "buf_obs",
+        "buf_actions", "buf_values", "buf_log_probs", "buf_episode_starts", "buf_rewards", "last_values", "mean_out")] + [
+        ("clip_obs", C.c_double), ("epsilon", C.c_double), ("seed", C.c_uint64), ("env_id_offset", C.c_int64),
+        ("gamma", C.c_float), ("iteration", C.c_int32), ("step", C.c_int32), ("n_steps", C.c_int32), ("n", C.c_int32),
+        ("values_only", C.c_int32), ("deterministic", C.c_int32)]
 
 
 class QsStatePtrs(C.Structure):
@@ -156,6 +172,10 @@ EXPORTS = {
     "qs_obs_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 8),
     "qs_ars_act": (C.c_int, [C.c_void_p] * 3 + [C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_float, C.c_int,
                              C.c_int, C.c_int, C.POINTER(QsArsArch), C.c_void_p, C.c_int, C.c_void_p]),
+    "qs_ppo_act": (C.c_int, [C.POINTER(QsPpoArgs), C.POINTER(QsPpoArch), C.c_void_p]),
+    "qs_ppo_reward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_double] * 3 +
+                      [C.c_void_p] * 5),
+    "qs_ppo_gae": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_double, C.c_double] + [C.c_void_p] * 3),
     "qs_launch_count": (C.c_int64, []),
 }
 

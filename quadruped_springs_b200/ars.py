@@ -165,14 +165,14 @@ class _SB3Pickler(pickle._Pickler):
         self.memoize(obj)
 
 
-def write_vecnormalize_pkl(path, state, num_envs, norm_obs=True, training=True):
+def write_vecnormalize_pkl(path, state, num_envs, norm_obs=True, training=True, norm_reward=False):
     """a `VecNormalize.save()`-shaped pickle of VecNormalizeTorch.state_dict() `state` (protocol 4)"""
     rms = lambda m, v, c: _RunningMeanStdState(mean=np.asarray(m, np.float64), var=np.asarray(v, np.float64), count=float(c))
     vn = _VecNormalizeState(
         obs_rms=rms(state["obs_mean"], state["obs_var"], state["obs_count"]),
         ret_rms=rms(state["ret_mean"], state["ret_var"], state["ret_count"]),
         clip_obs=float(state["clip_obs"]), clip_reward=float(state["clip_reward"]), gamma=float(state["gamma"]),
-        epsilon=float(state["epsilon"]), training=bool(training), norm_obs=bool(norm_obs), norm_reward=False,
+        epsilon=float(state["epsilon"]), training=bool(training), norm_obs=bool(norm_obs), norm_reward=bool(norm_reward),
         num_envs=int(num_envs), norm_obs_keys=None)
     buf = io.BytesIO()
     _SB3Pickler(buf, protocol=4).dump(vn)
